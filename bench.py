@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- cavity-force + Bussi step throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one 1M-particle (+1 photon) synthetic charged box:
 the cavity force (dipole reduce + per-particle force + photon force + energies) and the
@@ -31,6 +31,12 @@ larger than the 126 MB L2), so no step finds its inputs in L2.
 N > 1 (torchrun, one process per GPU): every rank runs an independent replica (BASELINE configs[2],
 no data-path collective; "scaling": "weak"); rank 0 reports the aggregate; the sharded and F(k,t)
 legs then use all N GPUs for ONE problem.
+
+--dump-outputs DIR writes what the last timed cavb200_step of rank 0 returned to its caller as float64
+.npy files (see dump_outputs), so that two builds run with the same arguments can be compared output
+for output: every input is generated from fixed seeds.  The velocities and the reservoir's cumulative
+energy carry every earlier step on the same handle and system, warm-up included, so two dumps are
+comparable only when --n-mol, --systems, --warmup and --steps all match.
 """
 from __future__ import annotations
 
@@ -375,6 +381,28 @@ class DeviceSystem:
         self.image = capi.DeviceArray.from_numpy(s.image)
         self.vel = capi.DeviceArray.from_numpy(s.vel)
         self.force = capi.DeviceArray((s.N, 4), np.float64)
+
+
+DUMP_ROWS = 1 << 19  # per-particle arrays of larger systems are dumped as this many rows: 2 x 16 MB
+
+
+def dump_outputs(out_dir, h, d, st):
+    """What the last cavb200_step handed its caller: the force array and the rescaled velocities of the system it ran
+    on, the energies, dipole and photon index (cavb200_force_read) and the thermostat record ke, alpha, instantaneous,
+    cumulative, err (cavb200_bussi_read).  A system of more than DUMP_ROWS particles contributes a fixed, seeded sample
+    of rows that always holds the last one (the photon of the bench's systems)."""
+    os.makedirs(out_dir, exist_ok=True)
+    force, vel = d.force.numpy(st), d.vel.numpy(st)
+    if d.N > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(d.N - 1, DUMP_ROWS - 1, replace=False))
+        rows = np.append(rows, d.N - 1)
+        force, vel = force[rows], vel[rows]
+    en, dip, ph = h.force_read(st)
+    bo = h.bussi_read(st)
+    out = {"force": force, "vel": vel, "energies": en, "dipole": dip, "photon_idx": [ph],
+           "bussi": [bo[k] for k in ("ke", "alpha", "instantaneous", "cumulative", "err")]}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 class Ctx:
@@ -749,6 +777,8 @@ def run_b200(args):
     m0 = sampler.mark()
     K = args.steps
     ms_fused, launches_fused = cx.timed(step, K, k0=W)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, h, systems[(W + K - 1) % len(systems)], st)
     ms_fused_hostpaced, _ = cx.timed(step, K, k0=W + K, gate=False)
     ms_sep, launches_sep = cx.timed(two_calls, K, k0=W)
     ms_sep_list, _ = cx.timed(lambda k: two_calls(k, gidx_range), K, k0=W)
@@ -1081,7 +1111,11 @@ def main():
     ap.add_argument("--no-fkt", action="store_true")
     ap.add_argument("--no-sharded", action="store_true")
     ap.add_argument("--no-small-n", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the B200 path (--impl b200)")
     # stdout carries the ONE JSON line and nothing else: native libraries write there too (NCCL prints its version
     # banner to fd 1 when the sharded leg creates its communicator), so fd 1 points at stderr while the run lasts and
     # the line goes to the real stdout at the end
