@@ -90,6 +90,8 @@ _SIGNATURES = {
     "cavb200_md_step_fused": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _u32, _dbl, _dbl, _dbl, _dbl, _u32, _PP, _u32, _u32, _BP,
                                         _vp]),
     "cavb200_nvt_step_two_rank1": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _u32, _dbl, _u32, _dbl, _u32, _u32, _vp]),
+    "cavb200_group_set": (C.c_int, [_vp, _vp, _u32, _u32, _vp]),
+    "cavb200_rank1_reindex": (C.c_int, [_vp, _vp, _u32, _u32, _vp]),
     "cavb200_track_open": (C.c_int, [_vp, _u32]),
     "cavb200_track_set_reference": (C.c_int, [_vp, _vp]),
     "cavb200_track_record": (C.c_int, [_vp, _u64, _vp, _u32, _vp]),
@@ -511,6 +513,17 @@ class Handle:
         check(self.lib.cavb200_nvt_step_two_rank1(self.h, _ptr(vel), _ptr(force_other), _ptr(charge), _ptr(pos), N, dt,
                                                   L_typeid & 0xFFFFFFFF, couplstr, group_first, n_group, stream),
               "cavb200_nvt_step_two_rank1")
+
+    # -- index-list groups and particle sorts ----------------------------------------------------
+    GROUP_MASK = 0xFFFFFFFF  # CAVB200_GROUP_MASK: pass as group_first to thermostat the mask of the last group_set
+
+    def group_set(self, group_idx, n, N, stream=None):
+        """Build the handle's group mask from the device index list group_idx (uint32[n]) of N particles (blocking)."""
+        check(self.lib.cavb200_group_set(self.h, _ptr(group_idx), n, N, stream), "cavb200_group_set")
+
+    def rank1_reindex(self, pos, N, L_typeid, stream=None):
+        """After a permutation of the particle arrays: move the photon index of the last rank-1 result (blocking)."""
+        check(self.lib.cavb200_rank1_reindex(self.h, _ptr(pos), N, L_typeid & 0xFFFFFFFF, stream), "cavb200_rank1_reindex")
 
     # -- device-side trackers (SURVEY.md 8f.4) --------------------------------------------------
     TRACK_FIELDS = ("timestep", "dx", "dy", "dz", "qx", "qy", "qz", "harmonic", "coupling", "dipole_self", "autocorr",

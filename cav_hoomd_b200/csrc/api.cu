@@ -194,6 +194,7 @@ int cavb200_destroy(cavb200_handle* h)
     cudaFree(h->stamps);
     cudaFree(h->rhok_partials);
     cudaFree(h->rhok_table);
+    cudaFree(h->group_mask);
     if (h->fault_host)
         cudaFreeHost(h->fault_host);
     free(h);

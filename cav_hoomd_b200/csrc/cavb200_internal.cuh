@@ -123,7 +123,8 @@ struct cavb200_handle
     int coop_supported;
     cavb::Partial* partials;          // MAX_PARTIALS records
     cavb::Scalars* scalars;           // 1 record
-    unsigned long long* counters;     // [2] hand-off epoch, [4] reduce-pass ticket, [8..] Final (variant 0), [32..] Final (rank-1)
+    unsigned long long* counters;     // [2] hand-off epoch, [4] reduce-pass ticket, [8..] Final (variant 0), [32..] Final (rank-1),
+                                      // [48] cavb200_group_set check word, [49..51] cavb200_rank1_reindex {first, count, ticket}
     uint64_t launches;
     uint64_t faults;                  // hand-off timeouts seen so far (each one switched the handle to cooperative launches)
     unsigned long long* fault_host;   // pinned + mapped: the word Scalars::fault points at
@@ -147,6 +148,11 @@ struct cavb200_handle
     double* rhok_partials;
     uint64_t rhok_partials_bytes;
     void* rhok_table; // device, (cos, sin)(2 pi e / 512) as double2 (rhok.cu)
+    // thermostatted group as a bit mask (cavb200_group_set), used by the window entry points with CAVB200_GROUP_MASK
+    uint32_t* group_mask;             // device, ceil(N / 32) words
+    uint64_t group_mask_words;        // allocated words
+    uint32_t group_n, group_N;        // members and particle count the mask was built for
+    int group_ready;                  // the last cavb200_group_set succeeded
     };
 
 namespace cavb

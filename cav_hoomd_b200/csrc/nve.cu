@@ -9,6 +9,8 @@
 //   k_net_force_add_rank1   what a net-force sum does with that rank-1 contribution
 //   k_md_one                step one with the NEXT force's dipole reduce inside (positions read once)
 //   k_md_fused              step two of step t-1 + step one of step t in ONE persistent launch (148 B/particle)
+//   ... <MASK>              the thermostatted group as the handle's bit mask instead of a window (cavb200_group_set)
+//   k_group_mask / k_photon_reindex   cavb200_group_set / cavb200_rank1_reindex (once per particle sort)
 #include "hotpath.cuh"
 
 #ifndef CAVB_NVT_CTAS_PER_SM
@@ -67,6 +69,17 @@ __device__ __forceinline__ void wrap_particle(double4& p, unsigned long long i, 
         }
     }
 
+// Membership of the thermostatted group: the window [lo, hi), or (MASK) bit i of the handle's group mask
+// (cavb200_group_set: ceil(N/32) words, bit i%32 of word i/32).  Every launch of these kernels has a block size and a
+// grid stride that are multiples of 32, so the lanes of a warp hold 32 consecutive indices and read ONE mask word, a
+// broadcast load: 4 B per 32 particles and pass.
+// (Written out at each test as `MASK ? in_mask(mask, i) : i >= lo && i < hi`: behind a helper function returning bool
+// the window test compiles to different, if equivalent, instructions.)
+__device__ __forceinline__ bool in_mask(const uint32_t* mask, unsigned long long i)
+    {
+    return (__ldg(mask + (i >> 5)) >> (i & 31)) & 1u;
+    }
+
 template<bool RANK1>
 __device__ __forceinline__ double4 kick_force(const double4* force, unsigned long long i, const Rank1In& r, const Final& fin)
     {
@@ -84,10 +97,10 @@ __device__ __forceinline__ double4 kick_force(const double4* force, unsigned lon
     return fc;
     }
 
-template<bool RANK1, bool WRAP>
+template<bool RANK1, bool WRAP, bool MASK>
 __global__ void __launch_bounds__(256)
     k_nvt_one(double4* pos, double4* vel, const double4* force, uint32_t N, double dt, BussiIn b, Scalars* scalars,
-              Rank1In r1, WrapIn w)
+              Rank1In r1, WrapIn w, const uint32_t* mask)
     {
     __shared__ double s_alpha;
     __shared__ Final s_fin;
@@ -125,7 +138,7 @@ __global__ void __launch_bounds__(256)
         double4 v = ld256(vel + i);
         const double4 f = kick_force<RANK1>(force, i, r1, s_fin);
         double4 p = ld256(pos + i);
-        if (i >= lo && i < hi)
+        if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
             {
             v.x = __dmul_rn(v.x, alpha);
             v.y = __dmul_rn(v.y, alpha);
@@ -150,10 +163,10 @@ __global__ void __launch_bounds__(256)
 
 // step two: all: v += dt/2 f/m, and sum m|v|^2 of the group on the way out; the last CTA to take a
 // ticket folds the CTA records (fixed order) and leaves KE in Scalars for the next step one.
-template<bool RANK1>
+template<bool RANK1, bool MASK>
 __global__ void __launch_bounds__(256)
     k_nvt_two(double4* vel, const double4* force, uint32_t N, double dt, BussiIn b, Partial* recs, Scalars* scalars,
-              unsigned long long* ticket, Rank1In r1)
+              unsigned long long* ticket, Rank1In r1, const uint32_t* mask)
     {
     __shared__ BlockScratch sc;
     __shared__ int s_last;
@@ -179,7 +192,7 @@ __global__ void __launch_bounds__(256)
         v.y = __dadd_rn(v.y, __dmul_rn(hm, f.y));
         v.z = __dadd_rn(v.z, __dmul_rn(hm, f.z));
         st256(vel + i, v);
-        if (i >= lo && i < hi)
+        if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
             a.ke += v.w * (v.x * v.x + v.y * v.y + v.z * v.z);
         }
     ForceIn f0 = {};
@@ -207,10 +220,11 @@ __global__ void __launch_bounds__(256)
 // (src/CavityForceCompute.cc:107-109,124) -- positions are never read a second time.  The last CTA to take a
 // ticket folds the CTA records and leaves the new Scalars / Final for step two.  One launch replaces
 // cavb200_nvt_step_one_rank1 + cavb200_force_rank1.
-template<bool WRAP>
+template<bool WRAP, bool MASK>
 __global__ void __launch_bounds__(256, 3)
     k_md_one(double4* pos, double4* vel, const double4* force_other, uint32_t N, double dt, BussiIn b, Scalars* scalars,
-             Rank1In r1, ForceIn fnew, Partial* recs, unsigned long long* ticket, Final* fin_out, WrapIn w)
+             Rank1In r1, ForceIn fnew, Partial* recs, unsigned long long* ticket, Final* fin_out, WrapIn w,
+             const uint32_t* mask)
     {
     __shared__ BlockScratch sc;
     __shared__ double s_alpha;
@@ -263,7 +277,7 @@ __global__ void __launch_bounds__(256, 3)
             f.y = __dadd_rn(fo.y, f.y);
             f.z = __dadd_rn(fo.z, f.z);
             }
-        if (i >= lo && i < hi)
+        if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
             {
             v.x = __dmul_rn(v.x, alpha);
             v.y = __dmul_rn(v.y, alpha);
@@ -312,11 +326,11 @@ __global__ void __launch_bounds__(256, 3)
 // pass, an L2 hit at 1M particles).  Structure of k_split_folder: 295 streaming CTAs, one folder CTA.
 //     streaming CTA:  pass 1 (v1 on the fly, KE) -> publish | take alpha | pass 2 (v2, r, dipole) -> publish
 //     folder CTA:     fold KE records -> alpha -> Final(K) | fold dipole records -> Scalars, Final for the next step
-template<int LB, int U2, bool WRAP>
+template<int LB, int U2, bool WRAP, bool MASK>
 __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
     k_md_fused(double4* pos, double4* vel, const double4* force_other, uint32_t N, double dt, BussiIn b, Rank1In r1,
                ForceIn fnew, Partial* recsF, Partial* recsB, Partial* finals, Scalars* scalars,
-               unsigned long long* epoch_ctr, Final* fin_out, WrapIn w)
+               unsigned long long* epoch_ctr, Final* fin_out, WrapIn w, const uint32_t* mask)
     {
     __shared__ BlockScratch sc;
     __shared__ Final s_fin;
@@ -398,9 +412,9 @@ __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
                          az = __dadd_rn(va.z, __dmul_rn(ha, fa.z));
             const double bx = __dadd_rn(vb.x, __dmul_rn(hb, fb.x)), by = __dadd_rn(vb.y, __dmul_rn(hb, fb.y)),
                          bz = __dadd_rn(vb.z, __dmul_rn(hb, fb.z));
-            if (i >= lo && i < hi)
+            if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
                 ke0 += va.w * (ax * ax + ay * ay + az * az);
-            if (i + stride >= lo && i + stride < hi)
+            if (MASK ? in_mask(mask, i + stride) : i + stride >= lo && i + stride < hi)
                 ke1 += vb.w * (bx * bx + by * by + bz * bz);
             }
         for (; i < N; i += stride)
@@ -415,7 +429,7 @@ __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
             const double ha = __ddiv_rn(half_dt, va.w);
             const double ax = __dadd_rn(va.x, __dmul_rn(ha, fa.x)), ay = __dadd_rn(va.y, __dmul_rn(ha, fa.y)),
                          az = __dadd_rn(va.z, __dmul_rn(ha, fa.z));
-            if (i >= lo && i < hi)
+            if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
                 ke0 += va.w * (ax * ax + ay * ay + az * az);
             }
         a.ke = ke0 + ke1;
@@ -443,7 +457,7 @@ __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
         v.x = __dadd_rn(v.x, __dmul_rn(hm, f.x));
         v.y = __dadd_rn(v.y, __dmul_rn(hm, f.y));
         v.z = __dadd_rn(v.z, __dmul_rn(hm, f.z));
-        if (i >= lo && i < hi)
+        if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
             {
             v.x = __dmul_rn(v.x, alpha);
             v.y = __dmul_rn(v.y, alpha);
@@ -543,6 +557,61 @@ __global__ void __launch_bounds__(256) k_nve(double4* pos, double4* vel, const d
             }
         }
     }
+
+// Group mask from an index list (the words were zeroed before the launch): bit idx[k] of the mask is set.  bad gets
+// bit 0 for an index >= N and bit 1 for an index that is listed twice (its bit was already set).
+__global__ void __launch_bounds__(256) k_group_mask(const uint32_t* idx, uint32_t n, uint32_t N, uint32_t* mask,
+                                                    unsigned long long* bad)
+    {
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long k = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride)
+        {
+        const uint32_t i = __ldg(idx + k);
+        if (i >= N)
+            {
+            atomicOr(bad, 1ull);
+            continue;
+            }
+        const uint32_t bit = 1u << (i & 31);
+        if (atomicOr(mask + (i >> 5), bit) & bit)
+            atomicOr(bad, 2ull);
+        }
+    }
+
+// After the particle arrays were permuted: the lowest index whose type id (low 32 bits of pos.w) is L_typeid, and how
+// many such particles there are, in s[0] / s[1] (set to ~0 / 0 before the launch).  The last CTA to take the ticket
+// s[2] patches the rank-1 Final record when there is exactly one: photon_local is the only field of it that depends on
+// the order of the particles (Dq, F_L and the energies are sums and products over the whole system).
+__global__ void __launch_bounds__(256) k_photon_reindex(const double4* pos, uint32_t N, uint32_t L_typeid,
+                                                        unsigned long long* s, Final* fin)
+    {
+    unsigned int first = NO_INDEX, cnt = 0;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride)
+        if (__double2loint(__ldg(&pos[i].w)) == (int)L_typeid)
+            {
+            first = first < (unsigned int)i ? first : (unsigned int)i;
+            cnt++;
+            }
+    first = __reduce_min_sync(0xffffffffu, first);
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if ((threadIdx.x & 31) == 0 && cnt)
+        {
+        atomicMin(s, (unsigned long long)first);
+        atomicAdd(s + 1, (unsigned long long)cnt);
+        }
+    __syncthreads();
+    if (threadIdx.x == 0)
+        {
+        __threadfence();
+        const bool last = atom_acq_rel_add_u64(s + 2, 1ull) == (unsigned long long)gridDim.x - 1;
+        if (last && ld_relaxed_u64(s + 1) == 1ull)
+            {
+            fin->photon_local = (long long)ld_relaxed_u64(s);
+            fin->many_L = 0;
+            }
+        }
+    }
     } // namespace cavb
 
 using namespace cavb;
@@ -621,6 +690,20 @@ __global__ void __launch_bounds__(256) k_net_force_add_rank1(double4* net, uint3
 
 static bool mis32(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 31) != 0; }
 
+// The thermostatted group of the window entry points: [group_first, group_first + n_group), or, with group_first ==
+// CAVB200_GROUP_MASK, the mask of the last cavb200_group_set (which must have been made for n_group members of N
+// particles).  Returns false for a group that does not fit; *mask is the mask to pass to the kernels, or NULL.
+static bool group_ok(const cavb200_handle* h, uint32_t N, uint32_t group_first, uint32_t n_group, const uint32_t** mask)
+    {
+    *mask = nullptr;
+    if (group_first != CAVB200_GROUP_MASK)
+        return (unsigned long long)group_first + n_group <= N;
+    if (!h->group_ready || n_group != h->group_n || N != h->group_N)
+        return false;
+    *mask = h->group_mask;
+    return true;
+    }
+
 static int fill_rank1(cavb200_handle* h, Rank1In& r, const double* charge, const double* pos, uint32_t L_typeid,
                       double couplstr)
     {
@@ -641,7 +724,8 @@ static int nvt_one(cavb200_handle* h, double* pos, double* vel, const double* fo
                    uint32_t group_first, uint32_t n_group, const cavb200_bussi_args* bussi, const Rank1In* r1, void* stream,
                    const WrapIn* w = nullptr)
     {
-    if (!pos || !vel || (!force && !r1) || (unsigned long long)group_first + n_group > N)
+    const uint32_t* mask;
+    if (!pos || !vel || (!force && !r1) || !group_ok(h, N, group_first, n_group, &mask))
         return (int)cudaErrorInvalidValue;
     if (mis32(pos) || mis32(vel) || mis32(force))
         return (int)cudaErrorMisalignedAddress;
@@ -657,14 +741,27 @@ static int nvt_one(cavb200_handle* h, double* pos, double* vel, const double* fo
     cudaStream_t cs = (cudaStream_t)stream;
     double4 *p4 = (double4*)pos, *v4 = (double4*)vel;
     const double4* f4 = (const double4*)force;
-    if (r1 && w)
-        k_nvt_one<true, true><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, *r1, *w);
+    const Rank1In r = r1 ? *r1 : Rank1In();
+    const WrapIn wr = w ? *w : WrapIn();
+    if (mask)
+        {
+        if (r1 && w)
+            k_nvt_one<true, true, true><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, mask);
+        else if (r1)
+            k_nvt_one<true, false, true><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, mask);
+        else if (w)
+            k_nvt_one<false, true, true><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, mask);
+        else
+            k_nvt_one<false, false, true><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, mask);
+        }
+    else if (r1 && w)
+        k_nvt_one<true, true, false><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, nullptr);
     else if (r1)
-        k_nvt_one<true, false><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, *r1, WrapIn());
+        k_nvt_one<true, false, false><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, nullptr);
     else if (w)
-        k_nvt_one<false, true><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, Rank1In(), *w);
+        k_nvt_one<false, true, false><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, nullptr);
     else
-        k_nvt_one<false, false><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, Rank1In(), WrapIn());
+        k_nvt_one<false, false, false><<<grid, 256, 0, cs>>>(p4, v4, f4, N, dt, b, h->scalars, r, wr, nullptr);
     CAVB_CHECK(cudaGetLastError());
     h->launches += 1;
     return 0;
@@ -673,7 +770,8 @@ static int nvt_one(cavb200_handle* h, double* pos, double* vel, const double* fo
 static int nvt_two(cavb200_handle* h, double* vel, const double* force, uint32_t N, double dt, uint32_t group_first,
                    uint32_t n_group, const Rank1In* r1, void* stream)
     {
-    if (!vel || (!force && !r1) || (unsigned long long)group_first + n_group > N)
+    const uint32_t* mask;
+    if (!vel || (!force && !r1) || !group_ok(h, N, group_first, n_group, &mask))
         return (int)cudaErrorInvalidValue;
     if (mis32(vel) || mis32(force))
         return (int)cudaErrorMisalignedAddress;
@@ -685,12 +783,18 @@ static int nvt_two(cavb200_handle* h, double* vel, const double* force, uint32_t
     if (cap > (unsigned long long)MAX_PARTIALS)
         cap = MAX_PARTIALS;
     const int grid = (int)(want < cap ? want : cap);
-    if (r1)
-        k_nvt_two<true><<<grid, 256, 0, (cudaStream_t)stream>>>((double4*)vel, (const double4*)force, N, dt, b, h->partials,
-                                                                h->scalars, h->counters + 4, *r1);
+    cudaStream_t cs = (cudaStream_t)stream;
+    double4* v4 = (double4*)vel;
+    const double4* f4 = (const double4*)force;
+    const Rank1In r = r1 ? *r1 : Rank1In();
+    if (r1 && mask)
+        k_nvt_two<true, true><<<grid, 256, 0, cs>>>(v4, f4, N, dt, b, h->partials, h->scalars, h->counters + 4, r, mask);
+    else if (r1)
+        k_nvt_two<true, false><<<grid, 256, 0, cs>>>(v4, f4, N, dt, b, h->partials, h->scalars, h->counters + 4, r, nullptr);
+    else if (mask)
+        k_nvt_two<false, true><<<grid, 256, 0, cs>>>(v4, f4, N, dt, b, h->partials, h->scalars, h->counters + 4, r, mask);
     else
-        k_nvt_two<false><<<grid, 256, 0, (cudaStream_t)stream>>>((double4*)vel, (const double4*)force, N, dt, b,
-                                                                 h->partials, h->scalars, h->counters + 4, Rank1In());
+        k_nvt_two<false, false><<<grid, 256, 0, cs>>>(v4, f4, N, dt, b, h->partials, h->scalars, h->counters + 4, r, nullptr);
     CAVB_CHECK(cudaGetLastError());
     h->launches += 1;
     return 0;
@@ -789,7 +893,8 @@ static int md_step_one_impl(cavb200_handle* h, double* pos, double* vel, const d
         return (int)cudaErrorInvalidValue;
     if (N == 0)
         return 0;
-    if (!pos || !vel || !charge || !image || !params || (unsigned long long)group_first + n_group > N)
+    const uint32_t* mask;
+    if (!pos || !vel || !charge || !image || !params || !group_ok(h, N, group_first, n_group, &mask))
         return (int)cudaErrorInvalidValue;
     if (mis32(pos) || mis32(vel) || mis32(force_other) || (reinterpret_cast<uintptr_t>(image) & 3))
         return (int)cudaErrorMisalignedAddress;
@@ -822,17 +927,25 @@ static int md_step_one_impl(cavb200_handle* h, double* pos, double* vel, const d
     const int grid = (int)(want < cap ? want : cap);
     WrapIn w = WrapIn();
     if (wrap)
-        {
         if (const int rcw = make_wrap(w, const_cast<int32_t*>(image), Lx, Ly, Lz))
             return rcw;
-        k_md_one<true><<<grid, 256, 0, (cudaStream_t)stream>>>((double4*)pos, (double4*)vel, (const double4*)force_other, N,
-                                                                dt, b, h->scalars, r, fnew, h->partials, h->counters + 4,
-                                                                const_cast<Final*>(rank1_final(h)), w);
-        }
+    cudaStream_t cs = (cudaStream_t)stream;
+    double4* p4 = (double4*)pos;
+    double4* v4 = (double4*)vel;
+    const double4* fo4 = (const double4*)force_other;
+    Final* fin_out = const_cast<Final*>(rank1_final(h));
+    if (wrap && mask)
+        k_md_one<true, true><<<grid, 256, 0, cs>>>(p4, v4, fo4, N, dt, b, h->scalars, r, fnew, h->partials, h->counters + 4,
+                                                   fin_out, w, mask);
+    else if (wrap)
+        k_md_one<true, false><<<grid, 256, 0, cs>>>(p4, v4, fo4, N, dt, b, h->scalars, r, fnew, h->partials, h->counters + 4,
+                                                    fin_out, w, nullptr);
+    else if (mask)
+        k_md_one<false, true><<<grid, 256, 0, cs>>>(p4, v4, fo4, N, dt, b, h->scalars, r, fnew, h->partials, h->counters + 4,
+                                                    fin_out, w, mask);
     else
-        k_md_one<false><<<grid, 256, 0, (cudaStream_t)stream>>>((double4*)pos, (double4*)vel, (const double4*)force_other, N,
-                                                                 dt, b, h->scalars, r, fnew, h->partials, h->counters + 4,
-                                                                 const_cast<Final*>(rank1_final(h)), w);
+        k_md_one<false, false><<<grid, 256, 0, cs>>>(p4, v4, fo4, N, dt, b, h->scalars, r, fnew, h->partials,
+                                                     h->counters + 4, fin_out, w, nullptr);
     CAVB_CHECK(cudaGetLastError());
     h->launches += 1;
     return 0;
@@ -865,7 +978,8 @@ static int md_step_fused_impl(cavb200_handle* h, double* pos, double* vel, const
         return (int)cudaErrorInvalidValue;
     if (N == 0)
         return 0;
-    if (!pos || !vel || !charge || !image || !params || (unsigned long long)group_first + n_group > N)
+    const uint32_t* mask;
+    if (!pos || !vel || !charge || !image || !params || !group_ok(h, N, group_first, n_group, &mask))
         return (int)cudaErrorInvalidValue;
     if (mis32(pos) || mis32(vel) || mis32(force_other) || (reinterpret_cast<uintptr_t>(image) & 3))
         return (int)cudaErrorMisalignedAddress;
@@ -904,12 +1018,18 @@ static int md_step_fused_impl(cavb200_handle* h, double* pos, double* vel, const
     switch (h->tune.md_shape)
         {
     case 1:
-        kern = wrap ? (const void*)k_md_fused<384, 1, true> : (const void*)k_md_fused<384, 1, false>;
+        if (mask)
+            kern = wrap ? (const void*)k_md_fused<384, 1, true, true> : (const void*)k_md_fused<384, 1, false, true>;
+        else
+            kern = wrap ? (const void*)k_md_fused<384, 1, true, false> : (const void*)k_md_fused<384, 1, false, false>;
         threads = 384;
         per_sm_want = 2;
         break;
     default: // folder CTA alone on its SM
-        kern = wrap ? (const void*)k_md_fused<768, 1, true> : (const void*)k_md_fused<768, 1, false>;
+        if (mask)
+            kern = wrap ? (const void*)k_md_fused<768, 1, true, true> : (const void*)k_md_fused<768, 1, false, true>;
+        else
+            kern = wrap ? (const void*)k_md_fused<768, 1, true, false> : (const void*)k_md_fused<768, 1, false, false>;
         threads = 768;
         per_sm_want = 1;
         break;
@@ -935,7 +1055,7 @@ static int md_step_fused_impl(cavb200_handle* h, double* pos, double* vel, const
     Scalars* sca = h->scalars;
     unsigned long long* ctr = h->counters + 2;
     Final* fin_out = const_cast<Final*>(rank1_final(h));
-    void* args[] = {&p4, &v4, &fo4, &N, &dt, &b, &r, &fnew, &recsF, &recsB, &finals, &sca, &ctr, &fin_out, &w};
+    void* args[] = {&p4, &v4, &fo4, &N, &dt, &b, &r, &fnew, &recsF, &recsB, &finals, &sca, &ctr, &fin_out, &w, &mask};
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(threads);
@@ -998,4 +1118,71 @@ extern "C" int cavb200_net_force_add_rank1(cavb200_handle* h, double* net_force,
     CAVB_CHECK(cudaGetLastError());
     h->launches += 1;
     return 0;
+    }
+
+// ---- index-list groups ---------------------------------------------------------------------------------------------
+extern "C" int cavb200_group_set(cavb200_handle* h, const uint32_t* group_idx, uint32_t n, uint32_t N, void* stream)
+    {
+    if (!h || (n && !group_idx))
+        return (int)cudaErrorInvalidValue;
+    if (reinterpret_cast<uintptr_t>(group_idx) & 3)
+        return (int)cudaErrorMisalignedAddress;
+    h->group_ready = 0;
+    const unsigned long long words = ((unsigned long long)N + 31) / 32;
+    if (words > h->group_mask_words)
+        {
+        cudaFree(h->group_mask);
+        h->group_mask = nullptr;
+        h->group_mask_words = 0;
+        CAVB_CHECK(cudaMalloc((void**)&h->group_mask, words * sizeof(uint32_t)));
+        h->group_mask_words = words;
+        }
+    cudaStream_t cs = (cudaStream_t)stream;
+    unsigned long long* bad = h->counters + 48;
+    CAVB_CHECK(cudaMemsetAsync(bad, 0, sizeof(unsigned long long), cs));
+    if (words)
+        CAVB_CHECK(cudaMemsetAsync(h->group_mask, 0, words * sizeof(uint32_t), cs));
+    if (n)
+        {
+        const unsigned long long want = ((unsigned long long)n + 255) / 256;
+        const unsigned long long cap = (unsigned long long)h->num_sms * 8;
+        k_group_mask<<<(int)(want < cap ? want : cap), 256, 0, cs>>>(group_idx, n, N, h->group_mask, bad);
+        CAVB_CHECK(cudaGetLastError());
+        h->launches += 1;
+        }
+    unsigned long long flags = 0;
+    CAVB_CHECK(cudaMemcpyAsync(&flags, bad, sizeof(flags), cudaMemcpyDeviceToHost, cs));
+    CAVB_CHECK(cudaStreamSynchronize(cs));
+    if (flags)
+        return (int)cudaErrorInvalidValue; // an index >= N (bit 0) or one listed twice (bit 1)
+    h->group_n = n;
+    h->group_N = N;
+    h->group_ready = 1;
+    return 0;
+    }
+
+extern "C" int cavb200_rank1_reindex(cavb200_handle* h, const double* pos, uint32_t N, uint32_t L_typeid, void* stream)
+    {
+    if (!h || (N && !pos))
+        return (int)cudaErrorInvalidValue;
+    if (mis32(pos))
+        return (int)cudaErrorMisalignedAddress;
+    if (N == 0)
+        return 0;
+    cudaStream_t cs = (cudaStream_t)stream;
+    unsigned long long* sc = h->counters + 49; // {first, count, ticket}
+    CAVB_CHECK(cudaMemsetAsync(sc, 0xFF, sizeof(unsigned long long), cs));
+    CAVB_CHECK(cudaMemsetAsync(sc + 1, 0, 2 * sizeof(unsigned long long), cs));
+    const unsigned long long want = ((unsigned long long)N + 255) / 256;
+    const unsigned long long cap = (unsigned long long)h->num_sms * 8;
+    k_photon_reindex<<<(int)(want < cap ? want : cap), 256, 0, cs>>>(reinterpret_cast<const double4*>(pos), N, L_typeid, sc,
+                                                                     const_cast<Final*>(rank1_final(h)));
+    CAVB_CHECK(cudaGetLastError());
+    h->launches += 1;
+    unsigned long long found[2];
+    CAVB_CHECK(cudaMemcpyAsync(found, sc, sizeof(found), cudaMemcpyDeviceToHost, cs));
+    CAVB_CHECK(cudaStreamSynchronize(cs));
+    // several 'L' particles: which of them F_L was computed for is not recorded, so the first one by index after a sort
+    // need not be it
+    return found[1] > 1 ? (int)cudaErrorNotSupported : 0;
     }

@@ -15,6 +15,7 @@
 #ifndef HOOMD_SHIM_CORE_H
 #define HOOMD_SHIM_CORE_H
 
+#include <algorithm>
 #include <array>
 #include <cmath>
 #include <cstdint>
@@ -219,6 +220,37 @@ class BoxDim
     Scalar3 m_L;
     };
 
+//! The part of Nano::Signal<void()> the plugin uses: connect / disconnect a member function of an object; emit() calls
+//! the connected slots in the order they were connected.
+class Signal
+    {
+    public:
+    template<class T, void (T::*M)()> void connect(T* obj) { m_slots.push_back({obj, &thunk<T, M>}); }
+    template<class T, void (T::*M)()> void disconnect(T* obj)
+        {
+        for (size_t k = 0; k < m_slots.size(); k++)
+            if (m_slots[k].obj == obj && m_slots[k].fn == &thunk<T, M>)
+                {
+                m_slots.erase(m_slots.begin() + (std::ptrdiff_t)k);
+                return;
+                }
+        }
+    void emit()
+        {
+        const std::vector<Slot> slots = m_slots;
+        for (const Slot& sl : slots)
+            sl.fn(sl.obj);
+        }
+    private:
+    template<class T, void (T::*M)()> static void thunk(void* o) { (static_cast<T*>(o)->*M)(); }
+    struct Slot
+        {
+        void* obj;
+        void (*fn)(void*);
+        };
+    std::vector<Slot> m_slots;
+    };
+
 class ParticleData
     {
     public:
@@ -230,6 +262,9 @@ class ParticleData
         ArrayHandle<unsigned int> h_tag(m_tag, access_location::host, access_mode::overwrite);
         for (unsigned int i = 0; i < N; i++)
             h_tag.data[i] = i;
+        m_rtag.resize(N);
+        for (unsigned int i = 0; i < N; i++)
+            m_rtag[i] = i;
         }
     unsigned int getN() const { return m_N; }
     unsigned int getNGlobal() const { return m_N; }
@@ -242,6 +277,39 @@ class ParticleData
     const GPUArray<Scalar>& getCharges() const { return m_charge; }
     const GPUArray<int3>& getImages() const { return m_image; }
     const GPUArray<unsigned int>& getTags() const { return m_tag; }
+    //! current index of the particle with tag `tag`
+    unsigned int getRTag(unsigned int tag) const { return m_rtag.at(tag); }
+    //! emitted after the particle arrays were reordered (HOOMD's particle sorter); slots connect with
+    //! getParticleSortSignal().connect<Class, &Class::slot>(this)
+    Signal& getParticleSortSignal() { return m_sort_signal; }
+    //! shim only, what HOOMD's sorter does: the particle now at index j is the one that was at order[j].  Every array
+    //! that is indexed by particle moves with it (net force included); then the signal is emitted, and the groups
+    //! rebuild their index lists from it.
+    void sortParticles(const std::vector<unsigned int>& order)
+        {
+        if (order.size() != m_N)
+            throw std::runtime_error("hoomd_shim: sortParticles needs one index per particle");
+        std::vector<char> seen(m_N, 0);
+        for (unsigned int o : order)
+            {
+            if (o >= m_N || seen[o])
+                throw std::runtime_error("hoomd_shim: sortParticles needs a permutation");
+            seen[o] = 1;
+            }
+        permute(m_pos, order);
+        permute(m_vel, order);
+        permute(m_accel, order);
+        permute(m_charge, order);
+        permute(m_image, order);
+        permute(m_net_force, order);
+        permute(m_tag, order);
+            {
+            ArrayHandle<unsigned int> h_tag(m_tag, access_location::host, access_mode::read);
+            for (unsigned int i = 0; i < m_N; i++)
+                m_rtag[h_tag.data[i]] = i;
+            }
+        m_sort_signal.emit();
+        }
     //! sum of all ForceCompute arrays, formed by the integrator between step one and step two
     const GPUArray<Scalar4>& getNetForce() const { return m_net_force; }
     unsigned int getNTypes() const { return (unsigned int)m_types.size(); }
@@ -254,6 +322,13 @@ class ParticleData
         }
     std::shared_ptr<ExecutionConfiguration> getExecConf() const { return m_exec; }
     private:
+    template<class T> void permute(const GPUArray<T>& a, const std::vector<unsigned int>& order)
+        {
+        ArrayHandle<T> h(a, access_location::host, access_mode::readwrite);
+        const std::vector<T> old(h.data, h.data + m_N);
+        for (unsigned int j = 0; j < m_N; j++)
+            h.data[j] = old[order[j]];
+        }
     unsigned int m_N;
     BoxDim m_box;
     std::vector<std::string> m_types;
@@ -264,6 +339,8 @@ class ParticleData
     GPUArray<int3> m_image;
     GPUArray<unsigned int> m_tag;
     GPUArray<Scalar4> m_net_force;
+    std::vector<unsigned int> m_rtag;
+    Signal m_sort_signal;
     };
 
 class SystemDefinition
@@ -341,31 +418,50 @@ class VariantConstant : public Variant
     Scalar m_v;
     };
 
-//! ParticleGroup: an index list into the particle arrays (tags == indices in the shim)
+//! ParticleGroup: a set of particle tags and its index list into the particle arrays.  The shim's particles start with
+//! tag == index, so the list is the members as given until the first sort; after a sort it is rebuilt in ascending
+//! index order (HOOMD rebuilds it on its sort signal).
 class ParticleGroup
     {
     public:
     ParticleGroup(std::shared_ptr<SystemDefinition> sysdef, const std::vector<unsigned int>& members)
-        : m_sysdef(sysdef), m_members(members),
+        : m_sysdef(sysdef), m_members(members), m_index(members),
           m_idx(members.size(), sysdef->getParticleData()->getExecConf()), m_tdof(0), m_rdof(0)
         {
         ArrayHandle<unsigned int> h(m_idx, access_location::host, access_mode::overwrite);
         for (size_t i = 0; i < members.size(); i++)
             h.data[i] = members[i];
+        m_sysdef->getParticleData()->getParticleSortSignal().connect<ParticleGroup, &ParticleGroup::slotParticleSort>(this);
         }
+    ~ParticleGroup()
+        {
+        m_sysdef->getParticleData()->getParticleSortSignal().disconnect<ParticleGroup, &ParticleGroup::slotParticleSort>(this);
+        }
+    ParticleGroup(const ParticleGroup&) = delete;
+    ParticleGroup& operator=(const ParticleGroup&) = delete;
     unsigned int getNumMembers() const { return (unsigned int)m_members.size(); }
     unsigned int getNumMembersGlobal() const { return (unsigned int)m_members.size(); }
     unsigned int getMemberTag(unsigned int i) const { return m_members[i]; }
-    unsigned int getMemberIndex(unsigned int i) const { return m_members[i]; }
+    unsigned int getMemberIndex(unsigned int i) const { return m_index[i]; }
     const GPUArray<unsigned int>& getIndexArray() const { return m_idx; }
     //! true when the members are exactly first, first+1, ... (lets kernels skip the gather)
     bool isContiguous(unsigned int& first) const
         {
-        first = m_members.empty() ? 0 : m_members[0];
-        for (size_t i = 0; i < m_members.size(); i++)
-            if (m_members[i] != first + i)
+        first = m_index.empty() ? 0 : m_index[0];
+        for (size_t i = 0; i < m_index.size(); i++)
+            if (m_index[i] != first + i)
                 return false;
         return true;
+        }
+    void slotParticleSort()
+        {
+        auto pdata = m_sysdef->getParticleData();
+        for (size_t i = 0; i < m_members.size(); i++)
+            m_index[i] = pdata->getRTag(m_members[i]);
+        std::sort(m_index.begin(), m_index.end());
+        ArrayHandle<unsigned int> h(m_idx, access_location::host, access_mode::overwrite);
+        for (size_t i = 0; i < m_index.size(); i++)
+            h.data[i] = m_index[i];
         }
     Scalar getTranslationalDOF() const { return m_tdof; }
     Scalar getRotationalDOF() const { return m_rdof; }
@@ -373,7 +469,8 @@ class ParticleGroup
     void setRotationalDOF(Scalar d) { m_rdof = d; }
     private:
     std::shared_ptr<SystemDefinition> m_sysdef;
-    std::vector<unsigned int> m_members;
+    std::vector<unsigned int> m_members; // tags
+    std::vector<unsigned int> m_index;   // their current indices (the host copy of m_idx)
     GPUArray<unsigned int> m_idx;
     Scalar m_tdof, m_rdof;
     };

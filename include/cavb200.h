@@ -264,6 +264,25 @@ int cavb200_md_step_fused_wrap(cavb200_handle* h, double* pos, double* vel, cons
                                const cavb200_params* params, uint32_t group_first, uint32_t n_group,
                                const cavb200_bussi_args* bussi, void* stream);
 
+/* ---- index-list groups and particle sorts -------------------------------------------------------
+ * HOOMD hands a group out as an index list, and its particle sorter permutes the particle arrays.
+ *   cavb200_group_set      builds the handle's group mask (one bit per particle, ceil(N/32) words) from the device
+ *                          index list group_idx[n] of a system of N particles.  Blocking: returns
+ *                          cudaErrorInvalidValue for an index >= N or an index listed twice (no mask is then set).
+ *                          Call it once per change of the list, not per step.
+ *   CAVB200_GROUP_MASK     passed as `group_first` to cavb200_nvt_step_one(_wrap), _two, _one_rank1(_wrap),
+ *                          _two_rank1, cavb200_md_step_one(_wrap) and cavb200_md_step_fused(_wrap): the thermostatted
+ *                          group is that mask.  `n_group` and `N` must be the n and N of the last cavb200_group_set,
+ *                          else (or without one) the call returns cudaErrorInvalidValue.  A mask that holds the range
+ *                          [first, first + n) gives bit-identical results to group_first = first.
+ *   cavb200_rank1_reindex  after a permutation of the particle arrays: finds the particle of type L_typeid (low 32 bits
+ *                          of pos.w) again and moves the photon index of the last rank-1 result there, so that the
+ *                          next rank-1 kick gives F_L to the photon.  Dq, F_L and the energies do not depend on the
+ *                          order.  Blocking; cudaErrorNotSupported when more than one particle has that type. */
+#define CAVB200_GROUP_MASK 0xFFFFFFFFu
+int cavb200_group_set(cavb200_handle* h, const uint32_t* group_idx, uint32_t n, uint32_t N, void* stream);
+int cavb200_rank1_reindex(cavb200_handle* h, const double* pos, uint32_t N, uint32_t L_typeid, void* stream);
+
 /* ---- device-side trackers (SURVEY.md 8f.4) ------------------------------------------------------
  * Replace the per-step cpu_local_snapshot of the reference's trackers (reference
  * src/cavitymd/analysis.py:188,234 AutocorrelationTracker / DipoleAutocorrelation, :1327

@@ -74,7 +74,15 @@ PYBIND11_MODULE(_hoomd_shim, m)
                  return out;
              })
         .def("getVelocities", [](ParticleData& p) { return fetch<Scalar4, 4>(p.getVelocities(), p.getN()); })
-        .def("getPositions", [](ParticleData& p) { return fetch<Scalar4, 4>(p.getPositions(), p.getN()); });
+        .def("getPositions", [](ParticleData& p) { return fetch<Scalar4, 4>(p.getPositions(), p.getN()); })
+        .def("getTags",
+             [](ParticleData& p)
+             {
+                 ArrayHandle<unsigned int> h(p.getTags(), access_location::host, access_mode::read);
+                 return std::vector<unsigned int>(h.data, h.data + p.getN());
+             })
+        // what HOOMD's particle sorter does (ShimCore.h): the particle now at index j is the one that was at order[j]
+        .def("sortParticles", &ParticleData::sortParticles);
 
     py::class_<SystemDefinition, std::shared_ptr<SystemDefinition>>(m, "SystemDefinition")
         .def(py::init<std::shared_ptr<ParticleData>, uint16_t>(), py::arg("pdata"), py::arg("seed") = 0)

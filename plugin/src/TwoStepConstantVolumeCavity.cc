@@ -12,7 +12,8 @@ TwoStepConstantVolumeCavity::TwoStepConstantVolumeCavity(std::shared_ptr<SystemD
                                                          std::shared_ptr<cavitymd::CavityForceComputeGPU> cavity,
                                                          const std::string& mode)
     : IntegrationMethodTwoStep(sysdef, group), m_thermostat(thermostat), m_source(nullptr), m_cavity(cavity),
-      m_handle(nullptr), m_started(false), m_pending(false)
+      m_handle(nullptr), m_started(false), m_pending(false), m_index_list(false), m_group_stale(true), m_use_mask(false),
+      m_first(0), m_group_n(0), m_group_N(0), m_photon_stale(false)
     {
     if (!m_exec_conf->isCUDAEnabled())
         throw std::runtime_error("TwoStepConstantVolumeCavity requires a GPU execution configuration (no CPU fallback)");
@@ -43,10 +44,13 @@ TwoStepConstantVolumeCavity::TwoStepConstantVolumeCavity(std::shared_ptr<SystemD
         m_source->adoptHandle(m_handle);
     if (m_cavity && m_mode != STORED)
         m_cavity->useHandle(m_handle, m_mode == RANK1 ? 1 : 2);
+    m_pdata->getParticleSortSignal().connect<TwoStepConstantVolumeCavity, &TwoStepConstantVolumeCavity::slotParticleSort>(this);
     }
 
 TwoStepConstantVolumeCavity::~TwoStepConstantVolumeCavity()
     {
+    m_pdata->getParticleSortSignal().disconnect<TwoStepConstantVolumeCavity, &TwoStepConstantVolumeCavity::slotParticleSort>(
+        this);
     if (m_source)
         m_source->adoptHandle(nullptr);
     if (m_cavity && m_mode != STORED)
@@ -88,13 +92,81 @@ void TwoStepConstantVolumeCavity::window(unsigned int& first, unsigned int& n)
                 throw std::runtime_error("TwoStepConstantVolumeCavity: the thermostatted group must be a contiguous index range");
     }
 
+void TwoStepConstantVolumeCavity::setIndexListGroup(bool on)
+    {
+    m_index_list = on;
+    m_group_stale = true;
+    }
+
+void TwoStepConstantVolumeCavity::slotParticleSort()
+    {
+    m_group_stale = true;
+    m_photon_stale = true;
+    }
+
+uint32_t TwoStepConstantVolumeCavity::photonTypeId() const
+    {
+    try
+        {
+        return m_pdata->getTypeByName("L");
+        }
+    catch (...)
+        {
+        return 0xFFFFFFFFu;
+        }
+    }
+
+void TwoStepConstantVolumeCavity::group(unsigned int& first, unsigned int& n)
+    {
+    if (!m_index_list)
+        {
+        window(first, n);
+        return;
+        }
+    n = m_group->getNumMembers();
+    const unsigned int N = m_pdata->getN();
+    if (m_group_stale || n != m_group_n || N != m_group_N)
+        {
+        bool contiguous = true;
+            {
+            ArrayHandle<unsigned int> h_idx(m_group->getIndexArray(), access_location::host, access_mode::read);
+            m_first = n ? h_idx.data[0] : 0;
+            for (unsigned int j = 0; j < n && contiguous; j++)
+                contiguous = h_idx.data[j] == m_first + j;
+            }
+        m_use_mask = !contiguous;
+        if (m_use_mask)
+            {
+            ArrayHandle<unsigned int> d_idx(m_group->getIndexArray(), access_location::device, access_mode::read);
+            check(cavb200_group_set(m_handle, d_idx.data, n, N, nullptr), "cavb200_group_set");
+            }
+        m_group_n = n;
+        m_group_N = N;
+        m_group_stale = false;
+        }
+    first = m_use_mask ? CAVB200_GROUP_MASK : m_first;
+    }
+
+void TwoStepConstantVolumeCavity::reindexPhoton(uint32_t L_typeid)
+    {
+    // the rank-1 kicks give F_L to the particle at the photon index of the last result, which a sort has moved
+    if (!m_photon_stale || m_mode == STORED)
+        return;
+    ArrayHandle<Scalar4> d_pos(m_pdata->getPositions(), access_location::device, access_mode::read);
+    check(cavb200_rank1_reindex(m_handle, reinterpret_cast<const double*>(d_pos.data), m_pdata->getN(), L_typeid, nullptr),
+          "cavb200_rank1_reindex (the rank-1 modes follow a particle sort with one particle of type 'L' only)");
+    m_photon_stale = false;
+    }
+
 void TwoStepConstantVolumeCavity::integrateStepOne(uint64_t timestep)
     {
     const unsigned int N = m_pdata->getN();
     if (N == 0)
         return;
     unsigned int first = 0, n = 0;
-    window(first, n);
+    group(first, n);
+    const uint32_t L_typeid = photonTypeId();
+    reindexPhoton(L_typeid);
     const Scalar3 L = m_pdata->getGlobalBox().getL();
     cavb200_bussi_args args = {};
     const cavb200_bussi_args* bussi = nullptr;
@@ -116,16 +188,14 @@ void TwoStepConstantVolumeCavity::integrateStepOne(uint64_t timestep)
     if (!m_started)
         {
         // the first alpha needs KE(v(t0)): one reduce pass, once (afterwards step two leaves the next KE on the device)
-        check(cavb200_bussi_ke(m_handle, vel, nullptr, first, n, nullptr), "cavb200_bussi_ke");
+        if (first == CAVB200_GROUP_MASK)
+            {
+            ArrayHandle<unsigned int> d_idx(m_group->getIndexArray(), access_location::device, access_mode::read);
+            check(cavb200_bussi_ke(m_handle, vel, d_idx.data, 0, n, nullptr), "cavb200_bussi_ke");
+            }
+        else
+            check(cavb200_bussi_ke(m_handle, vel, nullptr, first, n, nullptr), "cavb200_bussi_ke");
         m_started = true;
-        }
-    uint32_t L_typeid = 0xFFFFFFFFu;
-    try
-        {
-        L_typeid = m_pdata->getTypeByName("L");
-        }
-    catch (...)
-        {
         }
     switch (m_mode)
         {
@@ -165,7 +235,9 @@ void TwoStepConstantVolumeCavity::integrateStepTwo(uint64_t timestep)
         return;
         }
     unsigned int first = 0, n = 0;
-    window(first, n);
+    group(first, n);
+    const uint32_t L_typeid = photonTypeId();
+    reindexPhoton(L_typeid);
     ArrayHandle<Scalar4> d_vel(m_pdata->getVelocities(), access_location::device, access_mode::readwrite);
     ArrayHandle<Scalar4> d_net(m_pdata->getNetForce(), access_location::device, access_mode::read);
     double* vel = reinterpret_cast<double*>(d_vel.data);
@@ -177,14 +249,6 @@ void TwoStepConstantVolumeCavity::integrateStepTwo(uint64_t timestep)
         }
     ArrayHandle<Scalar4> d_pos(m_pdata->getPositions(), access_location::device, access_mode::read);
     ArrayHandle<Scalar> d_charge(m_pdata->getCharges(), access_location::device, access_mode::read);
-    uint32_t L_typeid = 0xFFFFFFFFu;
-    try
-        {
-        L_typeid = m_pdata->getTypeByName("L");
-        }
-    catch (...)
-        {
-        }
     check(cavb200_nvt_step_two_rank1(m_handle, vel, net, d_charge.data, reinterpret_cast<const double*>(d_pos.data), N,
                                      m_deltaT, L_typeid, m_cavity->params().couplstr, first, n, nullptr),
           "cavb200_nvt_step_two_rank1");
@@ -196,19 +260,13 @@ void TwoStepConstantVolumeCavity::flush()
         return;
     const unsigned int N = m_pdata->getN();
     unsigned int first = 0, n = 0;
-    window(first, n);
+    group(first, n);
+    const uint32_t L_typeid = photonTypeId();
+    reindexPhoton(L_typeid); // the deferred kick forms the rank-1 force from the last result
     ArrayHandle<Scalar4> d_vel(m_pdata->getVelocities(), access_location::device, access_mode::readwrite);
     ArrayHandle<Scalar4> d_net(m_pdata->getNetForce(), access_location::device, access_mode::read);
     ArrayHandle<Scalar4> d_pos(m_pdata->getPositions(), access_location::device, access_mode::read);
     ArrayHandle<Scalar> d_charge(m_pdata->getCharges(), access_location::device, access_mode::read);
-    uint32_t L_typeid = 0xFFFFFFFFu;
-    try
-        {
-        L_typeid = m_pdata->getTypeByName("L");
-        }
-    catch (...)
-        {
-        }
     check(cavb200_nvt_step_two_rank1(m_handle, reinterpret_cast<double*>(d_vel.data), reinterpret_cast<const double*>(d_net.data),
                                      d_charge.data, reinterpret_cast<const double*>(d_pos.data), N, m_deltaT, L_typeid,
                                      m_cavity->params().couplstr, first, n, nullptr),
@@ -229,6 +287,8 @@ void export_TwoStepConstantVolumeCavity(pybind11::module& m)
              py::arg("sysdef"), py::arg("group"), py::arg("thermostat"), py::arg("cavity_force"), py::arg("mode") = "rank1")
         .def("flush", &TwoStepConstantVolumeCavity::flush)
         .def_property_readonly("mode", &TwoStepConstantVolumeCavity::getMode)
+        .def_property("index_list_group", &TwoStepConstantVolumeCavity::getIndexListGroup,
+                      &TwoStepConstantVolumeCavity::setIndexListGroup)
         .def("getLaunchCount", &TwoStepConstantVolumeCavity::getLaunchCount);
     }
     } // namespace detail

@@ -18,9 +18,14 @@
 //                      (cavb200_md_step_fused_wrap: second half kick, KE -> alpha, rescale, first half kick, drift, wrap,
 //                      dipole reduce of the new positions).  Between steps the velocities are half a kick behind;
 //                      flush() completes them (call it before anything reads velocities, and at the end of a run).
-// Restrictions (checked, stated in INTEGRATION.md): every particle of the system is integrated by this method and the
-// thermostatted group must be a contiguous index range [first, first + n) -- e.g. all molecular particles with the
-// photon first or last; point particles only; single rank.
+// Thermostatted group: with index_list_group = false (default) it must be a contiguous index range [first, first + n)
+// -- e.g. all molecular particles with the photon first or last -- and the kernels take that window.  With
+// index_list_group = true any group is accepted: a contiguous list still takes the window, any other list becomes the
+// handle's bit mask (cavb200_group_set, CAVB200_GROUP_MASK), rebuilt when HOOMD's particle sorter has reordered the
+// particles or the group / particle count changed.  In either case a sort (getParticleSortSignal) also moves the photon
+// index of the last rank-1 result (cavb200_rank1_reindex) in the rank1 and one_launch modes, before the next launch.
+// Restrictions (checked, stated in INTEGRATION.md): every particle of the system is integrated by this method; point
+// particles only; single rank; with the sorter on, one particle of type 'L' in the rank-1 modes.
 #ifndef CAVB200_TWO_STEP_CONSTANT_VOLUME_CAVITY_H
 #define CAVB200_TWO_STEP_CONSTANT_VOLUME_CAVITY_H
 
@@ -50,9 +55,16 @@ class PYBIND11_EXPORT TwoStepConstantVolumeCavity : public IntegrationMethodTwoS
     void flush();
     std::string getMode() const;
     unsigned long long getLaunchCount() const { return cavb200_launch_count(m_handle); }
+    bool getIndexListGroup() const { return m_index_list; }
+    void setIndexListGroup(bool on);
+    //! HOOMD's particle sort signal: the mask and the photon index are rebuilt before the next launch
+    void slotParticleSort();
 
     private:
     void window(unsigned int& first, unsigned int& n);
+    void group(unsigned int& first, unsigned int& n);
+    void reindexPhoton(uint32_t L_typeid);
+    uint32_t photonTypeId() const;
     void check(int err, const char* what) const;
     enum Mode { STORED = 0, RANK1 = 1, ONE_LAUNCH = 2 };
     std::shared_ptr<Thermostat> m_thermostat;
@@ -62,6 +74,12 @@ class PYBIND11_EXPORT TwoStepConstantVolumeCavity : public IntegrationMethodTwoS
     Mode m_mode;
     bool m_started;   //!< the kinetic energy of the initial velocities has been put on the device
     bool m_pending;   //!< one_launch: a second half kick is outstanding
+    bool m_index_list;     //!< index_list_group: any group, as a mask when it is not a contiguous range
+    bool m_group_stale;    //!< index_list_group: the window / mask must be rebuilt before the next launch
+    bool m_use_mask;       //!< index_list_group: the group is the handle's mask (else the window at m_first)
+    unsigned int m_first;  //!< index_list_group: first index of a contiguous group
+    unsigned int m_group_n, m_group_N; //!< members and particle count the window / mask was built for
+    bool m_photon_stale;   //!< particles were sorted since the last rank-1 result was formed
     };
 
 namespace detail
