@@ -52,15 +52,10 @@ int check_fault(cavb200_handle* h)
     h->faults += 1;
     return (int)cudaErrorLaunchTimeout;
     }
-    } // namespace cavb
-
-namespace
-    {
-inline bool misaligned(const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
 
 int fill_force(ForceIn& f, const double* pos, const double* charge, const int32_t* image, double* force, uint32_t N,
                double Lx, double Ly, double Lz, uint32_t L_typeid, const cavb200_params* p, uint64_t index_offset,
-               bool need_force = true)
+               bool need_force)
     {
     if (!pos || !charge || !image || (need_force && !force) || !p)
         return (int)cudaErrorInvalidValue;
@@ -81,7 +76,10 @@ int fill_force(ForceIn& f, const double* pos, const double* charge, const int32_
     fill_force_constants(f);
     return 0;
     }
+    } // namespace cavb
 
+namespace
+    {
 int fill_bussi(BussiIn& b, double* vel, const uint32_t* gidx, uint32_t first, uint32_t n, const cavb200_bussi_args* a,
                int rescale)
     {

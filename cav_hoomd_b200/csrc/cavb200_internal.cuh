@@ -389,6 +389,12 @@ struct BussiIn
     };
 
 void fill_force_constants(ForceIn& f);
+inline bool misaligned(const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
+// ForceIn of one call from the entry point's arguments (api.cu): cudaErrorInvalidValue for a NULL pointer or params,
+// cudaErrorMisalignedAddress for a pointer off its alignment (pos, force 32 B; charge 8 B; image 4 B)
+int fill_force(ForceIn& f, const double* pos, const double* charge, const int32_t* image, double* force, uint32_t N,
+               double Lx, double Ly, double Lz, uint32_t L_typeid, const cavb200_params* p, uint64_t index_offset,
+               bool need_force = true);
 // device slot of the Final record cavb200_force_rank1 leaves for the rank-1 consumers (nve.cu); apart
 // from the variant-0 slot at counters + 8, which every reduce-only launch overwrites
 struct Final;
