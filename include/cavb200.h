@@ -209,7 +209,8 @@ int cavb200_nvt_step_one_wrap(cavb200_handle* h, double* pos, double* vel, const
  *   cavb200_force_rank1      cavb200_force without the force array: dipole reduce (52 B/particle read,
  *                            nothing written per particle); energies / dipole / photon index as
  *                            cavb200_force_read; Dq, F_L stay on the device for the consumers below.
- *   cavb200_rank1_read       Dq[2], F_L[3] (photon force, :203-207), photon index, number of 'L' particles.
+ *   cavb200_rank1_read       Dq[2], F_L[3] (photon force, :203-207), photon index, number of 'L' particles
+ *                            (a schedule that merges per-CTA records reports any number above one as 2).
  *   cavb200_net_force_add_rank1   net_force[i] += F_i formed from charge_i: what HOOMD's net-force sum
  *                            (Integrator::computeNetForceGPU, upstream) would do with this contribution.
  *                            The photon gets F_L; further 'L' particles get 0 (pos is only read, for the
