@@ -96,7 +96,7 @@ struct Tuning
     int small_n;         // calls over at most this many particles run as ONE CTA with no inter-CTA hand-off (0: off)
     int cluster_n;       // ... and, for calls that include the force, up to this many as ONE thread-block cluster of 16 CTAs:
                          //     hardware barrier instead of polled records (0: off; with a cluster of 8, half as many)
-    int rhok_threads;    // k_rhok CTA size: 128 or 256; 0 = by the number of wave vectors
+    int rhok_threads;    // k_rhok CTA size: 128 or 256; any other value (0 included) means 256
     int cluster_ctas;    // CTAs of that cluster (16 = non-portable size; the launcher falls back to 8 if the device refuses it)
     };
 

@@ -498,23 +498,29 @@ static int rhok_launch(cavb200_handle* h, const double* pos, uint32_t stride, ui
                             ? h->tune.rhok_threads
                             : RHOK_CTA;
     const uint32_t tiles = (N + RHOK_TILE - 1) / RHOK_TILE;
-    const uint32_t P = rhok_slices(tiles, T, 2u * (uint32_t)h->num_sms);
-    const int direct = (P == 1);
-    double* target = rho;
-    if (!direct)
+    const uint32_t slots = 2u * (uint32_t)h->num_sms;
+    // grid y is at most 65535: frames go in chunks of that many, each with its own slice count.  Chunks after the first
+    // start at offset pointers (frame_stride doubles -- floats on the float32 path, whose pointer travels as a double*
+    // -- per frame, 2K doubles of rho per frame), so the kernels never see more than one chunk.  Consecutive chunks reuse
+    // the workspace in stream order: k_rhok touches it only after pdl_wait(), i.e. after the previous fold has finished.
+    constexpr uint32_t TCHUNK = 65535;
+    uint64_t need = 0;
+    for (uint32_t t0 = 0; t0 < T; t0 += TCHUNK)
         {
-        const uint64_t need = sizeof(double) * 2ull * K * T * P;
-        if (h->rhok_partials_bytes < need)
-            {
-            // growing the workspace is the one place a call may synchronise (first call / larger batch)
-            CAVB_CHECK(cudaStreamSynchronize(s));
-            cudaFree(h->rhok_partials);
-            h->rhok_partials = nullptr;
-            h->rhok_partials_bytes = 0;
-            CAVB_CHECK(cudaMalloc((void**)&h->rhok_partials, need));
-            h->rhok_partials_bytes = need;
-            }
-        target = h->rhok_partials;
+        const uint32_t Tc = (T - t0) < TCHUNK ? (T - t0) : TCHUNK;
+        const uint32_t P = rhok_slices(tiles, Tc, slots);
+        if (P > 1 && sizeof(double) * 2ull * K * Tc * P > need)
+            need = sizeof(double) * 2ull * K * Tc * P;
+        }
+    if (h->rhok_partials_bytes < need)
+        {
+        // growing the workspace is the one place a call may synchronise (first call / larger batch)
+        CAVB_CHECK(cudaStreamSynchronize(s));
+        cudaFree(h->rhok_partials);
+        h->rhok_partials = nullptr;
+        h->rhok_partials_bytes = 0;
+        CAVB_CHECK(cudaMalloc((void**)&h->rhok_partials, need));
+        h->rhok_partials_bytes = need;
         }
     cudaLaunchAttribute pdl_attr;
     pdl_attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -524,43 +530,51 @@ static int rhok_launch(cavb200_handle* h, const double* pos, uint32_t stride, ui
 #define RHOK_KB 4
 #endif
     constexpr int KB = RHOK_KB;
-    for (uint32_t k0 = 0; k0 < K; k0 += (uint32_t)threads * KB)
+    for (uint32_t t0 = 0; t0 < T; t0 += TCHUNK)
         {
-        const uint32_t Ks = (K - k0) < (uint32_t)threads * KB ? (K - k0) : (uint32_t)threads * KB;
-        const uint32_t KQ = (Ks + KB - 1) / KB;
-        const uint32_t groups = (uint32_t)threads / KQ;
-        // table | two tile buffers (32 KB; the fold of the particle groups reuses them: 2 * groups * KQ * KB doubles <= 16 KB)
-        const size_t smem = sizeof(double2) * RHOK_TAB * RHOK_REP + sizeof(double4) * 2 * RHOK_TILE;
-        (void)groups;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(P, T);
-        cfg.blockDim = dim3(threads);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = s;
-        cfg.attrs = &pdl_attr;
-        cfg.numAttrs = h->tune.pdl ? 1 : 0;
-        unsigned long long fs = frame_stride;
-        const double2* tabp = (const double2*)h->rhok_table;
-        int direct_i = direct;
-        void* args[] = {(void*)&pos, (void*)&stride, (void*)&fs,    (void*)&N, (void*)&kvec,     (void*)&k0,
-                        (void*)&Ks,  (void*)&K,      (void*)&target, (void*)&P, (void*)&direct_i, (void*)&tabp};
-        CAVB_CHECK(cudaLaunchKernelExC(&cfg, stride == RHOK_F32 ? (const void*)k_rhok<KB, true> : (const void*)k_rhok<KB, false>,
-                                       args));
-        h->launches += 1;
-        }
-    if (!direct)
-        {
-        const unsigned long long pairs = (unsigned long long)T * K;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned int)((pairs * 32 + 255) / 256));
-        cfg.blockDim = dim3(256);
-        cfg.stream = s;
-        cfg.attrs = &pdl_attr;
-        cfg.numAttrs = h->tune.pdl ? 1 : 0;
-        const double* part = target;
-        void* args[] = {(void*)&part, (void*)&P, (void*)&K, (void*)&T, (void*)&rho};
-        CAVB_CHECK(cudaLaunchKernelExC(&cfg, (const void*)k_rhok_fold, args));
-        h->launches += 1;
+        const uint32_t Tc = (T - t0) < TCHUNK ? (T - t0) : TCHUNK;
+        const uint32_t P = rhok_slices(tiles, Tc, slots);
+        const int direct = (P == 1);
+        const double* pos_c = stride == RHOK_F32
+                                  ? reinterpret_cast<const double*>(reinterpret_cast<const float*>(pos) + t0 * frame_stride)
+                                  : pos + t0 * frame_stride;
+        double* rho_c = rho + 2ull * K * t0;
+        double* target = direct ? rho_c : h->rhok_partials;
+        for (uint32_t k0 = 0; k0 < K; k0 += (uint32_t)threads * KB)
+            {
+            const uint32_t Ks = (K - k0) < (uint32_t)threads * KB ? (K - k0) : (uint32_t)threads * KB;
+            // table | two tile buffers (32 KB; the fold of the particle groups reuses them: 2 * groups * KQ * KB doubles <= 16 KB)
+            const size_t smem = sizeof(double2) * RHOK_TAB * RHOK_REP + sizeof(double4) * 2 * RHOK_TILE;
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3(P, Tc);
+            cfg.blockDim = dim3(threads);
+            cfg.dynamicSmemBytes = smem;
+            cfg.stream = s;
+            cfg.attrs = &pdl_attr;
+            cfg.numAttrs = h->tune.pdl ? 1 : 0;
+            unsigned long long fs = frame_stride;
+            const double2* tabp = (const double2*)h->rhok_table;
+            int direct_i = direct;
+            void* args[] = {(void*)&pos_c, (void*)&stride, (void*)&fs,     (void*)&N, (void*)&kvec,     (void*)&k0,
+                            (void*)&Ks,    (void*)&K,      (void*)&target, (void*)&P, (void*)&direct_i, (void*)&tabp};
+            CAVB_CHECK(cudaLaunchKernelExC(&cfg, stride == RHOK_F32 ? (const void*)k_rhok<KB, true> : (const void*)k_rhok<KB, false>,
+                                           args));
+            h->launches += 1;
+            }
+        if (!direct)
+            {
+            const unsigned long long pairs = (unsigned long long)Tc * K;
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3((unsigned int)((pairs * 32 + 255) / 256));
+            cfg.blockDim = dim3(256);
+            cfg.stream = s;
+            cfg.attrs = &pdl_attr;
+            cfg.numAttrs = h->tune.pdl ? 1 : 0;
+            const double* part = target;
+            void* args[] = {(void*)&part, (void*)&P, (void*)&K, (void*)&Tc, (void*)&rho_c};
+            CAVB_CHECK(cudaLaunchKernelExC(&cfg, (const void*)k_rhok_fold, args));
+            h->launches += 1;
+            }
         }
     return 0;
     }

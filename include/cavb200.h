@@ -313,7 +313,9 @@ int cavb200_track_read(cavb200_handle* h, double* out, uint32_t max_records, uin
  * rho[t][k] = sum_j exp(i kvec[k] . r_j(t)) over ALL N particles of frame t (wrapped positions),
  * the batched form of compute_density_field (reference src/cavitymd/analysis.py:34-47).
  * pos: T frames of N particles, `stride` doubles per particle (3 = xyz, 4 = HOOMD Scalar4),
- * frame t starts at pos + t*frame_stride doubles.  kvec: double[3*K] (device).
+ * frame t starts at pos + t*frame_stride doubles; frame_stride may exceed stride*N (frames cut from a larger
+ * buffer, rows after the N-th are never read) and must be a multiple of 4 for Scalar4 (which needs pos 32-byte aligned).
+ * T is limited only by uint32_t (frames are launched in chunks of at most 65535).  kvec: double[3*K] (device).
  * rho: double[2*K*T] (device), interleaved {re, im}.  Deterministic (fixed-order) reduction.
  * Each term exp(i x) is accurate to 2.4e-16 absolute per component (about 1 ulp of 1) for |x| < 2^20;
  * larger arguments, inf and nan go through the CUDA library's sincos.  The first call on a handle
@@ -323,7 +325,7 @@ int cavb200_rhok(cavb200_handle* h, const double* pos, uint32_t stride, uint64_t
 /* The same for float32 xyz positions, the way a GSD trajectory stores them (particles/position, Nx3 float32;
  * reference examples/05_advanced_run.py:1231-1246 writes the trajectory the analysis reads): 12 B/particle/frame
  * instead of 24-32 cross PCIe and HBM; the values are widened exactly, as NumPy does in np.dot(float32, float64)
- * (analysis.py:42).  frame t starts at pos_xyz + t*frame_stride FLOATS. */
+ * (analysis.py:42).  frame t starts at pos_xyz + t*frame_stride FLOATS (frame_stride may exceed 3*N; pos_xyz 4-byte aligned). */
 int cavb200_rhok_f32(cavb200_handle* h, const float* pos_xyz, uint64_t frame_stride, uint32_t N, uint32_t T,
                      const double* kvec, uint32_t K, double* rho, void* stream);
 /* F[o][l] = mean_k Re(rho[o][k] * conj(rho[o+l][k])) for origins o < n_origins, lags l < n_lags

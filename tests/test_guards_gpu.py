@@ -115,3 +115,48 @@ def test_guards_harness_steps(handle, n_mol):
     assert np.all(g["net"].get() == 0.0)                                                         # read-only here
     assert np.isfinite(g["pos"].get()[:, :3]).all() and np.isfinite(g["vel"].get()[:, :3]).all()
     assert handle.bussi_read()["err"] == 0.0
+
+
+# F(k,t): (N, T, K, rhok_threads, frame padding) -- direct multi-tile, folded, multi-slab, 128 threads
+RHOK_SHAPES = [(1537, 8000, 5, 256, 0), (1537, 8000, 5, 128, 1), (20001, 2, 64, 256, 0), (20001, 2, 1025, 256, 1),
+               (5000, 2, 2051, 128, 1), (100001, 3, 64, 128, 1)]
+
+
+@pytest.mark.parametrize("N,T,K,threads,pad", RHOK_SHAPES)
+@pytest.mark.parametrize("layout", ["xyz", "scalar4", "f32"])
+def test_guards_rhok(handle, N, T, K, threads, pad, layout):
+    """cavb200_rhok / _rhok_f32 write rho only inside its array; positions (padding between frames included) and the
+    wave vectors are unchanged byte for byte."""
+    rng = np.random.default_rng(N + T + K)
+    w, dt = (4, np.float64) if layout == "scalar4" else (3, np.float32 if layout == "f32" else np.float64)
+    fs = w * N + pad * (8 if layout == "scalar4" else 5 if layout == "xyz" else 1)
+    pos = np.full((T, fs), np.nan, dt)
+    pos[:, :w * N].reshape(T, N, w)[:, :, :3] = rng.uniform(-20, 20, size=(T, N, 3))
+    kvec = synth.fibonacci_sphere(max(K, 2))[:K]
+    g = {"pos": Guarded(pos), "kvec": Guarded(kvec), "rho": Guarded(np.full((T, K, 2), np.nan))}
+    handle.set_tuning(rhok_threads=threads)
+    if layout == "f32":
+        handle.rhok_f32(g["pos"].ptr, fs, N, T, g["kvec"].ptr, K, g["rho"].ptr)
+    else:
+        handle.rhok(g["pos"].ptr, w, fs, N, T, g["kvec"].ptr, K, g["rho"].ptr)
+    capi.sync()
+    handle.set_tuning(rhok_threads=0)
+    for k, a in g.items():
+        assert a.guards_intact(), f"guard of {k} overwritten"
+    assert np.array_equal(g["pos"].get().view(np.uint8), pos.view(np.uint8))
+    assert np.array_equal(g["kvec"].get().view(np.uint8), kvec.view(np.uint8))
+    assert np.isfinite(g["rho"].get()).all()
+
+
+@pytest.mark.parametrize("T,K,n_or,n_lag", [(12, 1, 8, 10), (1200, 64, 1000, 1000), (5, 4096, 9, 3)])
+def test_guards_fkt(handle, T, K, n_or, n_lag):
+    rng = np.random.default_rng(T + K)
+    rho = rng.standard_normal((T, K, 2)) * 100.0
+    g = {"rho": Guarded(rho), "out": Guarded(np.zeros((n_or, n_lag)))}
+    handle.fkt(g["rho"].ptr, T, K, n_or, n_lag, g["out"].ptr)
+    capi.sync()
+    for k, a in g.items():
+        assert a.guards_intact(), f"guard of {k} overwritten"
+    assert np.array_equal(g["rho"].get().view(np.uint8), rho.view(np.uint8))
+    o, l = np.meshgrid(np.arange(n_or), np.arange(n_lag), indexing="ij")
+    assert np.array_equal(np.isnan(g["out"].get()), o + l >= T)
