@@ -41,12 +41,23 @@ class BussiArgs(C.Structure):
                 ("r_normal", C.c_double), ("gamma_draw", C.c_double)]
 
 
+class LangevinArgs(C.Structure):
+    """struct cavb200_langevin_args: the cavity mode's Langevin bath, the draws of ONE step two (r uniform in [-1, 1])."""
+
+    _fields_ = [("gamma", C.c_double), ("kT", C.c_double), ("r", C.c_double * 3)]
+
+    @classmethod
+    def make(cls, gamma: float, kT: float, r) -> "LangevinArgs":
+        return cls(gamma, kT, (C.c_double * 3)(*[float(x) for x in r]))
+
+
 _vp = C.c_void_p
 _u32 = C.c_uint32
 _u64 = C.c_uint64
 _dbl = C.c_double
 _PP = C.POINTER(Params)
 _BP = C.POINTER(BussiArgs)
+_LP = C.POINTER(LangevinArgs)
 _dp = C.POINTER(C.c_double)
 
 _SIGNATURES = {
@@ -90,6 +101,13 @@ _SIGNATURES = {
     "cavb200_md_step_fused": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _u32, _dbl, _dbl, _dbl, _dbl, _u32, _PP, _u32, _u32, _BP,
                                         _vp]),
     "cavb200_nvt_step_two_rank1": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _u32, _dbl, _u32, _dbl, _u32, _u32, _vp]),
+    "cavb200_nvt_step_two_rank1_bath": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _u32, _dbl, _u32, _dbl, _u32, _u32, _LP, _vp]),
+    "cavb200_nvt_step_one_rank1_wrap_bath": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _u32, _dbl, _dbl, _dbl, _dbl, _u32,
+                                                       _dbl, _u32, _u32, _BP, _vp]),
+    "cavb200_md_step_one_wrap_bath": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _u32, _dbl, _dbl, _dbl, _dbl, _u32, _PP, _u32,
+                                                _u32, _BP, _vp]),
+    "cavb200_md_step_fused_wrap_bath": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _u32, _dbl, _dbl, _dbl, _dbl, _u32, _PP,
+                                                  _u32, _u32, _BP, _LP, _vp]),
     "cavb200_group_set": (C.c_int, [_vp, _vp, _u32, _u32, _vp]),
     "cavb200_rank1_reindex": (C.c_int, [_vp, _vp, _u32, _u32, _vp]),
     "cavb200_track_open": (C.c_int, [_vp, _u32]),
@@ -478,14 +496,19 @@ class Handle:
                                                    L_typeid & 0xFFFFFFFF, couplstr, stream),
               "cavb200_net_force_add_rank1")
 
+    # bath=: the cavity mode's Langevin bath (cavb200_*_bath).  Step one takes bath=True (the photon's kick adds the bath
+    # force the last step two stored); step two and the fused step take the LangevinArgs of the step two they perform.
+    # The bath entry points exist for the wrapped steps only.
     def nvt_step_one_rank1(self, pos, vel, force_other, charge, N, dt, L_typeid, couplstr, group_first, n_group,
-                           bussi=None, stream=None, image=None, box=None):
+                           bussi=None, stream=None, image=None, box=None, bath=False):
+        if bath and image is None:
+            raise ValueError("the photon bath comes with the box wrap only (image=, box=)")
         if image is not None:
-            check(self.lib.cavb200_nvt_step_one_rank1_wrap(self.h, _ptr(pos), _ptr(vel), _ptr(force_other), _ptr(charge),
-                                                           _ptr(image), N, dt, box[0], box[1], box[2], L_typeid & 0xFFFFFFFF,
-                                                           couplstr, group_first, n_group,
-                                                           C.byref(bussi) if bussi is not None else None, stream),
-                  "cavb200_nvt_step_one_rank1_wrap")
+            fn = self.lib.cavb200_nvt_step_one_rank1_wrap_bath if bath else self.lib.cavb200_nvt_step_one_rank1_wrap
+            check(fn(self.h, _ptr(pos), _ptr(vel), _ptr(force_other), _ptr(charge), _ptr(image), N, dt, box[0], box[1],
+                     box[2], L_typeid & 0xFFFFFFFF, couplstr, group_first, n_group,
+                     C.byref(bussi) if bussi is not None else None, stream),
+                  fn.__name__)
             return
         check(self.lib.cavb200_nvt_step_one_rank1(self.h, _ptr(pos), _ptr(vel), _ptr(force_other), _ptr(charge), N, dt,
                                                   L_typeid & 0xFFFFFFFF, couplstr, group_first, n_group,
@@ -493,23 +516,44 @@ class Handle:
               "cavb200_nvt_step_one_rank1")
 
     def md_step_one(self, pos, vel, force_other, charge, image, N, dt, box, L_typeid, params, group_first, n_group,
-                    bussi=None, stream=None, wrap=False):
-        fn = self.lib.cavb200_md_step_one_wrap if wrap else self.lib.cavb200_md_step_one
+                    bussi=None, stream=None, wrap=False, bath=False):
+        if bath and not wrap:
+            raise ValueError("the photon bath comes with the box wrap only (wrap=True)")
+        fn = self.lib.cavb200_md_step_one_wrap_bath if bath else (
+            self.lib.cavb200_md_step_one_wrap if wrap else self.lib.cavb200_md_step_one)
         check(fn(self.h, _ptr(pos), _ptr(vel), _ptr(force_other), _ptr(charge), _ptr(image), N,
                                            dt, box[0], box[1], box[2], L_typeid & 0xFFFFFFFF, C.byref(params), group_first,
                                            n_group, C.byref(bussi) if bussi is not None else None, stream),
               "cavb200_md_step_one")
 
     def md_step_fused(self, pos, vel, force_other, charge, image, N, dt, box, L_typeid, params, group_first, n_group,
-                      bussi=None, stream=None, wrap=False):
+                      bussi=None, stream=None, wrap=False, bath=None):
+        """bath: LangevinArgs of the deferred step two (the previous step's draws)."""
+        bussi_p = C.byref(bussi) if bussi is not None else None
+        if bath is not None:
+            if not wrap:
+                raise ValueError("the photon bath comes with the box wrap only (wrap=True)")
+            check(self.lib.cavb200_md_step_fused_wrap_bath(self.h, _ptr(pos), _ptr(vel), _ptr(force_other), _ptr(charge),
+                                                           _ptr(image), N, dt, box[0], box[1], box[2],
+                                                           L_typeid & 0xFFFFFFFF, C.byref(params), group_first, n_group,
+                                                           bussi_p, C.byref(bath), stream),
+                  "cavb200_md_step_fused_wrap_bath")
+            return
         fn = self.lib.cavb200_md_step_fused_wrap if wrap else self.lib.cavb200_md_step_fused
         check(fn(self.h, _ptr(pos), _ptr(vel), _ptr(force_other), _ptr(charge), _ptr(image), N,
                                              dt, box[0], box[1], box[2], L_typeid & 0xFFFFFFFF, C.byref(params),
-                                             group_first, n_group, C.byref(bussi) if bussi is not None else None, stream),
+                                             group_first, n_group, bussi_p, stream),
               "cavb200_md_step_fused")
 
     def nvt_step_two_rank1(self, vel, force_other, charge, pos, N, dt, L_typeid, couplstr, group_first, n_group,
-                           stream=None):
+                           stream=None, bath=None):
+        """bath: LangevinArgs of this step two."""
+        if bath is not None:
+            check(self.lib.cavb200_nvt_step_two_rank1_bath(self.h, _ptr(vel), _ptr(force_other), _ptr(charge), _ptr(pos),
+                                                           N, dt, L_typeid & 0xFFFFFFFF, couplstr, group_first, n_group,
+                                                           C.byref(bath), stream),
+                  "cavb200_nvt_step_two_rank1_bath")
+            return
         check(self.lib.cavb200_nvt_step_two_rank1(self.h, _ptr(vel), _ptr(force_other), _ptr(charge), _ptr(pos), N, dt,
                                                   L_typeid & 0xFFFFFFFF, couplstr, group_first, n_group, stream),
               "cavb200_nvt_step_two_rank1")

@@ -36,6 +36,24 @@ void fill_bussi_constants(BussiIn& b, const cavb200_bussi_args* a)
     const double K_bar = a->kT * a->dof / 2.0;              // :212
     b.den = (1.0 - b.c) * K_bar;
     }
+
+// HOOMD's TwoStepLangevin for one particle [HOOMD-upstream, not in the reference tree: restated from its definition]:
+// coeff = sqrt(6 gamma kT / dt), left to right, host libm; the three products coeff * r_c are formed here too, so the
+// device subtracts gamma v_c from bit-identical values
+int fill_bath(BathIn& b, const cavb200_handle* h, const cavb200_langevin_args* a, double dt)
+    {
+    b = BathIn();
+    b.bd = bath_slot(h);
+    if (!a)
+        return 0;
+    if (!(a->gamma >= 0.0) || !(a->kT >= 0.0) || !(dt > 0.0))
+        return (int)cudaErrorInvalidValue;
+    const double coeff = sqrt(6.0 * a->gamma * a->kT / dt);
+    b.gamma = a->gamma;
+    for (int c = 0; c < 3; c++)
+        b.cr[c] = coeff * a->r[c];
+    return 0;
+    }
     } // namespace cavb
 
 namespace cavb

@@ -124,7 +124,8 @@ struct cavb200_handle
     cavb::Partial* partials;          // MAX_PARTIALS records
     cavb::Scalars* scalars;           // 1 record
     unsigned long long* counters;     // [2] hand-off epoch, [4] reduce-pass ticket, [8..] Final (variant 0), [32..] Final (rank-1),
-                                      // [48] cavb200_group_set check word, [49..51] cavb200_rank1_reindex {first, count, ticket}
+                                      // [48] cavb200_group_set check word, [49..51] cavb200_rank1_reindex {first, count, ticket},
+                                      // [56..58] the photon's Langevin bath force bd[3] (double)
     uint64_t launches;
     uint64_t faults;                  // hand-off timeouts seen so far (each one switched the handle to cooperative launches)
     unsigned long long* fault_host;   // pinned + mapped: the word Scalars::fault points at
@@ -400,6 +401,20 @@ int fill_force(ForceIn& f, const double* pos, const double* charge, const int32_
 struct Final;
 inline const Final* rank1_final(const cavb200_handle* h) { return reinterpret_cast<const Final*>(h->counters + 32); }
 void fill_bussi_constants(BussiIn& b, const cavb200_bussi_args* a);
+// The cavity mode's Langevin bath as the harness kernels take it (nve.cu, BATH): bd = cr - gamma v of the photon, with
+// cr_c = coeff r_c and coeff = sqrt(6 gamma kT / dt) formed once on the host (api.cu fill_bath); bd points at the handle's
+// slot that holds the bath force of the last step two
+struct BathIn
+    {
+    double gamma;
+    double cr[3];
+    double* bd;
+    };
+// device slot of the bath force bd[3] (zero at cavb200_create)
+inline double* bath_slot(const cavb200_handle* h) { return reinterpret_cast<double*>(h->counters + 56); }
+// BathIn of one call: a = NULL gives the slot alone (step one reads the stored bd); cudaErrorInvalidValue for gamma < 0,
+// kT < 0 or dt <= 0
+int fill_bath(BathIn& b, const cavb200_handle* h, const cavb200_langevin_args* a, double dt);
 int launch_hotpath(cavb200_handle* h, const ForceIn* f, const BussiIn* b, cudaStream_t s);
 int cluster_kernels_init();
 int launch_shard_step(cavb200_handle* h, const ForceIn* f, const BussiIn* b, cudaStream_t s);

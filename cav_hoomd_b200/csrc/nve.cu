@@ -11,6 +11,7 @@
 //   k_md_fused              step two of step t-1 + step one of step t in ONE persistent launch (148 B/particle)
 //   ... <MASK>              the thermostatted group as the handle's bit mask instead of a window (cavb200_group_set)
 //   k_group_mask / k_photon_reindex   cavb200_group_set / cavb200_rank1_reindex (once per particle sort)
+//   ... <BATH>              the cavity mode's Langevin bath on the photon (cavb200_langevin_args, the *_bath entry points)
 #include "hotpath.cuh"
 
 #include <type_traits>
@@ -116,6 +117,40 @@ __device__ __forceinline__ double4 rank1_force(const double4* force_other, unsig
     return f;
     }
 
+// The cavity mode's Langevin bath (BATH), HOOMD's TwoStepLangevin on one particle [HOOMD-upstream, not in the reference
+// tree: restated from its definition]: the photon (the particle the rank-1 kick gives F_L to) kicks with
+// f = (f_other + F_L) + bd, bd_c = coeff r_c - gamma v_c formed in step two from the velocity before the kick.  HOOMD keeps
+// that sum as the acceleration, so the first half kick of the next step one adds the same bd, from the handle's slot.
+// Only the photon's thread reads gamma, cr and the slot: the streaming loops keep their registers.
+__device__ __forceinline__ bool is_photon(unsigned long long i, const Final& fin)
+    {
+    return fin.has_photon && (long long)i == fin.photon_local;
+    }
+// step one: f += the stored bd of the last step two
+__device__ __forceinline__ void add_stored_bath(double4& f, const BathIn& b)
+    {
+    f.x = __dadd_rn(f.x, b.bd[0]);
+    f.y = __dadd_rn(f.y, b.bd[1]);
+    f.z = __dadd_rn(f.z, b.bd[2]);
+    }
+// step two: bd = cr - gamma v; f += bd; STORE: bd goes to the slot
+template<bool STORE>
+__device__ __forceinline__ void add_new_bath(double4& f, const double4& v, const BathIn& b)
+    {
+    const double bx = __dadd_rn(b.cr[0], -__dmul_rn(b.gamma, v.x));
+    const double by = __dadd_rn(b.cr[1], -__dmul_rn(b.gamma, v.y));
+    const double bz = __dadd_rn(b.cr[2], -__dmul_rn(b.gamma, v.z));
+    f.x = __dadd_rn(f.x, bx);
+    f.y = __dadd_rn(f.y, by);
+    f.z = __dadd_rn(f.z, bz);
+    if (STORE)
+        {
+        b.bd[0] = bx;
+        b.bd[1] = by;
+        b.bd[2] = bz;
+        }
+    }
+
 template<bool RANK1>
 __device__ __forceinline__ double4 kick_force(const double4* force, unsigned long long i, const Rank1In& r, const Final& fin)
     {
@@ -174,10 +209,10 @@ __device__ __forceinline__ bool last_to_publish(Partial* recs, const BlockScratc
     return s_last;
     }
 
-template<bool RANK1, bool WRAP, bool MASK>
+template<bool RANK1, bool WRAP, bool MASK, bool BATH>
 __global__ void __launch_bounds__(256)
     k_nvt_one(double4* pos, double4* vel, const double4* force, uint32_t N, double dt, BussiIn b, Scalars* scalars,
-              Rank1In r1, WrapIn w, const uint32_t* mask)
+              Rank1In r1, WrapIn w, const uint32_t* mask, BathIn bath)
     {
     __shared__ double s_alpha;
     __shared__ Final s_fin;
@@ -194,7 +229,9 @@ __global__ void __launch_bounds__(256)
     for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride)
         {
         double4 v = ld256(vel + i);
-        const double4 f = kick_force<RANK1>(force, i, r1, s_fin);
+        double4 f = kick_force<RANK1>(force, i, r1, s_fin);
+        if (BATH && is_photon(i, s_fin))
+            add_stored_bath(f, bath);
         double4 p = ld256(pos + i);
         if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
             {
@@ -216,10 +253,10 @@ __global__ void __launch_bounds__(256)
 
 // step two: all: v += dt/2 f/m, and sum m|v|^2 of the group on the way out; the last CTA to take a
 // ticket folds the CTA records (fixed order) and leaves KE in Scalars for the next step one.
-template<bool RANK1, bool MASK>
+template<bool RANK1, bool MASK, bool BATH>
 __global__ void __launch_bounds__(256)
     k_nvt_two(double4* vel, const double4* force, uint32_t N, double dt, BussiIn b, Partial* recs, Scalars* scalars,
-              unsigned long long* ticket, Rank1In r1, const uint32_t* mask)
+              unsigned long long* ticket, Rank1In r1, const uint32_t* mask, BathIn bath)
     {
     __shared__ BlockScratch sc;
     __shared__ int s_last;
@@ -239,7 +276,9 @@ __global__ void __launch_bounds__(256)
     for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride)
         {
         double4 v = ld256(vel + i);
-        const double4 f = kick_force<RANK1>(force, i, r1, s_fin);
+        double4 f = kick_force<RANK1>(force, i, r1, s_fin);
+        if (BATH && is_photon(i, s_fin))
+            add_new_bath<true>(f, v, bath);
         half_kick(v, __ddiv_rn(__dmul_rn(0.5, dt), v.w), f);
         st256(vel + i, v);
         if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
@@ -262,11 +301,11 @@ __global__ void __launch_bounds__(256)
 // (src/CavityForceCompute.cc:107-109,124) -- positions are never read a second time.  The last CTA to take a
 // ticket folds the CTA records and leaves the new Scalars / Final for step two.  One launch replaces
 // cavb200_nvt_step_one_rank1 + cavb200_force_rank1.
-template<bool WRAP, bool MASK>
+template<bool WRAP, bool MASK, bool BATH>
 __global__ void __launch_bounds__(256, 3)
     k_md_one(double4* pos, double4* vel, const double4* force_other, uint32_t N, double dt, BussiIn b, Scalars* scalars,
              Rank1In r1, ForceIn fnew, Partial* recs, unsigned long long* ticket, Final* fin_out, WrapIn w,
-             const uint32_t* mask)
+             const uint32_t* mask, BathIn bath)
     {
     __shared__ BlockScratch sc;
     __shared__ double s_alpha;
@@ -290,7 +329,9 @@ __global__ void __launch_bounds__(256, 3)
         double4 p = ld256(pos + i);
         const double c = __ldg(fnew.charge + i);
         int3 im = load_image<WRAP>(w, fnew.image, i);
-        const double4 f = rank1_force(force_other, i, c, r1, s_fin);
+        double4 f = rank1_force(force_other, i, c, r1, s_fin);
+        if (BATH && is_photon(i, s_fin))
+            add_stored_bath(f, bath);
         if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
             {
             v.x = __dmul_rn(v.x, alpha);
@@ -327,11 +368,11 @@ __global__ void __launch_bounds__(256, 3)
 // pass, an L2 hit at 1M particles).  Structure of k_split_folder: 295 streaming CTAs, one folder CTA.
 //     streaming CTA:  pass 1 (v1 on the fly, KE) -> publish | take alpha | pass 2 (v2, r, dipole) -> publish
 //     folder CTA:     fold KE records -> alpha -> Final(K) | fold dipole records -> Scalars, Final for the next step
-template<int LB, int U2, bool WRAP, bool MASK>
+template<int LB, int U2, bool WRAP, bool MASK, bool BATH>
 __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
     k_md_fused(double4* pos, double4* vel, const double4* force_other, uint32_t N, double dt, BussiIn b, Rank1In r1,
                ForceIn fnew, Partial* recsF, Partial* recsB, Partial* finals, Scalars* scalars,
-               unsigned long long* epoch_ctr, Final* fin_out, WrapIn w, const uint32_t* mask)
+               unsigned long long* epoch_ctr, Final* fin_out, WrapIn w, const uint32_t* mask, BathIn bath)
     {
     __shared__ BlockScratch sc;
     __shared__ Final s_fin;
@@ -408,6 +449,10 @@ __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
                 add_other(fa, oa);
                 add_other(fb, ob);
                 }
+            if (BATH && is_photon(i, s_fin))
+                add_new_bath<false>(fa, va, bath); // the force pass 2 kicks the photon with: its KE term is the same
+            if (BATH && is_photon(i + stride, s_fin))
+                add_new_bath<false>(fb, vb, bath);
             const double ha = __ddiv_rn(half_dt, va.w), hb = __ddiv_rn(half_dt, vb.w);
             double4 a1 = va, b1 = vb;
             half_kick(a1, ha, fa);
@@ -423,6 +468,8 @@ __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
             double4 fa = force_of(i, __ldg(r1.charge + i), s_fin, r1.f);
             if (force_other)
                 add_other(fa, ld256(force_other + i));
+            if (BATH && is_photon(i, s_fin))
+                add_new_bath<false>(fa, va, bath);
             double4 a1 = va;
             half_kick(a1, __ddiv_rn(half_dt, va.w), fa);
             if (MASK ? in_mask(mask, i) : i >= lo && i < hi)
@@ -489,14 +536,19 @@ __global__ void __launch_bounds__(LB, LB == 384 ? 2 : 1)
             double4 fc = force_of(j, c[k], s_fin, r1.f);
             if (force_other)
                 add_other(fc, f[k]);
+            if (BATH && is_photon(j, s_fin))
+                add_new_bath<true>(fc, v[k], bath); // bd of the deferred step two: both half kicks, then the slot
             finish(j, v[k], p[k], c[k], im[k], fc);
             }
         }
     for (; i < N; i += stride)
         {
         const double c = __ldg(r1.charge + i);
-        const double4 fc = rank1_force(force_other, i, c, r1, s_fin);
-        finish(i, ld256(vel + i), ld256_na(pos + i), c, load_image<WRAP>(w, fnew.image, i), fc);
+        double4 fc = rank1_force(force_other, i, c, r1, s_fin);
+        const double4 v = ld256(vel + i);
+        if (BATH && is_photon(i, s_fin))
+            add_new_bath<true>(fc, v, bath);
+        finish(i, v, ld256_na(pos + i), c, load_image<WRAP>(w, fnew.image, i), fc);
         }
     block_merge<true, false>(a, fnew, sc);
     if (threadIdx.x == 0)
@@ -712,7 +764,7 @@ static int nve_launch(cavb200_handle* h, double* pos, double* vel, const double*
 
 static int nvt_one(cavb200_handle* h, double* pos, double* vel, const double* force, uint32_t N, double dt,
                    uint32_t group_first, uint32_t n_group, const cavb200_bussi_args* bussi, void* stream,
-                   const Rank1In* r1 = nullptr, const WrapIn* w = nullptr)
+                   const Rank1In* r1 = nullptr, const WrapIn* w = nullptr, bool bath = false)
     {
     if (!h)
         return (int)cudaErrorInvalidValue;
@@ -728,19 +780,24 @@ static int nvt_one(cavb200_handle* h, double* pos, double* vel, const double* fo
     const BussiIn b = harness_bussi(group_first, n_group, bussi);
     const Rank1In r = r1 ? *r1 : Rank1In();
     const WrapIn wr = w ? *w : WrapIn();
+    BathIn ba = BathIn();
+    if (bath)
+        fill_bath(ba, h, nullptr, dt); // the stored bd only
     const int grid = grid_for(h, N, CAVB_NVT_CTAS_PER_SM);
     with_flags(
-        [&](auto RANK1, auto WRAP, auto MASK)
+        [&](auto RANK1, auto WRAP, auto MASK, auto BATH)
         {
-            k_nvt_one<RANK1, WRAP, MASK><<<grid, 256, 0, (cudaStream_t)stream>>>(
-                (double4*)pos, (double4*)vel, (const double4*)force, N, dt, b, h->scalars, r, wr, mask);
+            if constexpr (!BATH || (RANK1 && WRAP)) // (the bath comes with the rank-1 wrap step only)
+                k_nvt_one<RANK1, WRAP, MASK, BATH><<<grid, 256, 0, (cudaStream_t)stream>>>(
+                    (double4*)pos, (double4*)vel, (const double4*)force, N, dt, b, h->scalars, r, wr, mask, ba);
         },
-        r1 != nullptr, w != nullptr, mask != nullptr);
+        r1 != nullptr, w != nullptr, mask != nullptr, bath);
     return launched(h);
     }
 
 static int nvt_two(cavb200_handle* h, double* vel, const double* force, uint32_t N, double dt, uint32_t group_first,
-                   uint32_t n_group, void* stream, const Rank1In* r1 = nullptr)
+                   uint32_t n_group, void* stream, const Rank1In* r1 = nullptr, bool bath = false,
+                   const cavb200_langevin_args* draws = nullptr)
     {
     if (!h)
         return (int)cudaErrorInvalidValue;
@@ -753,16 +810,20 @@ static int nvt_two(cavb200_handle* h, double* vel, const double* force, uint32_t
         return (int)cudaErrorInvalidValue;
     if (misaligned(vel, 32) || misaligned(force, 32))
         return (int)cudaErrorMisalignedAddress;
+    BathIn ba = BathIn();
+    if (bath && (!draws || fill_bath(ba, h, draws, dt)))
+        return (int)cudaErrorInvalidValue;
     const BussiIn b = harness_bussi(group_first, n_group, nullptr);
     const Rank1In r = r1 ? *r1 : Rank1In();
     const int grid = grid_for(h, N, CAVB_NVT_CTAS_PER_SM, true);
     with_flags(
-        [&](auto RANK1, auto MASK)
+        [&](auto RANK1, auto MASK, auto BATH)
         {
-            k_nvt_two<RANK1, MASK><<<grid, 256, 0, (cudaStream_t)stream>>>((double4*)vel, (const double4*)force, N, dt, b,
-                                                                          h->partials, h->scalars, h->counters + 4, r, mask);
+            if constexpr (!BATH || RANK1)
+                k_nvt_two<RANK1, MASK, BATH><<<grid, 256, 0, (cudaStream_t)stream>>>(
+                    (double4*)vel, (const double4*)force, N, dt, b, h->partials, h->scalars, h->counters + 4, r, mask, ba);
         },
-        r1 != nullptr, mask != nullptr);
+        r1 != nullptr, mask != nullptr, bath);
     return launched(h);
     }
 
@@ -833,6 +894,26 @@ extern "C" int cavb200_nvt_step_two_rank1(cavb200_handle* h, double* vel, const 
     return nvt_two(h, vel, force_other, N, dt, group_first, n_group, stream, &r);
     }
 
+extern "C" int cavb200_nvt_step_one_rank1_wrap_bath(cavb200_handle* h, double* pos, double* vel, const double* force_other,
+                                                    const double* charge, int32_t* image, uint32_t N, double dt, double Lx,
+                                                    double Ly, double Lz, uint32_t L_typeid, double couplstr,
+                                                    uint32_t group_first, uint32_t n_group,
+                                                    const cavb200_bussi_args* bussi, void* stream)
+    {
+    const Rank1In r = rank1_in(h, charge, pos, L_typeid, couplstr);
+    const WrapIn w = {image, Lx, Ly, Lz};
+    return nvt_one(h, pos, vel, force_other, N, dt, group_first, n_group, bussi, stream, &r, &w, true);
+    }
+
+extern "C" int cavb200_nvt_step_two_rank1_bath(cavb200_handle* h, double* vel, const double* force_other,
+                                               const double* charge, const double* pos, uint32_t N, double dt,
+                                               uint32_t L_typeid, double couplstr, uint32_t group_first, uint32_t n_group,
+                                               const cavb200_langevin_args* bath, void* stream)
+    {
+    const Rank1In r = rank1_in(h, charge, pos, L_typeid, couplstr);
+    return nvt_two(h, vel, force_other, N, dt, group_first, n_group, stream, &r, true, bath);
+    }
+
 // The arguments of k_md_one and k_md_fused
 struct MdArgs
     {
@@ -841,14 +922,18 @@ struct MdArgs
     Rank1In r;
     ForceIn fnew;
     WrapIn w;
+    BathIn bath;
     };
 
 static int md_args(MdArgs& a, cavb200_handle* h, const double* pos, const double* vel, const double* force_other,
-                   const double* charge, const int32_t* image, uint32_t N, double Lx, double Ly, double Lz,
+                   const double* charge, const int32_t* image, uint32_t N, double dt, double Lx, double Ly, double Lz,
                    uint32_t L_typeid, const cavb200_params* params, uint32_t group_first, uint32_t n_group,
-                   const cavb200_bussi_args* bussi, bool wrap)
+                   const cavb200_bussi_args* bussi, bool wrap, bool bath, const cavb200_langevin_args* draws)
     {
     if (!vel || !group_ok(h, N, group_first, n_group, &a.mask))
+        return (int)cudaErrorInvalidValue;
+    a.bath = BathIn();
+    if (bath && fill_bath(a.bath, h, draws, dt))
         return (int)cudaErrorInvalidValue;
     if (misaligned(vel, 32) || misaligned(force_other, 32))
         return (int)cudaErrorMisalignedAddress;
@@ -864,27 +949,28 @@ static int md_args(MdArgs& a, cavb200_handle* h, const double* pos, const double
 static int md_step_one_impl(cavb200_handle* h, double* pos, double* vel, const double* force_other,
                             const double* charge, const int32_t* image, uint32_t N, double dt, double Lx, double Ly,
                             double Lz, uint32_t L_typeid, const cavb200_params* params, uint32_t group_first,
-                            uint32_t n_group, const cavb200_bussi_args* bussi, void* stream, bool wrap)
+                            uint32_t n_group, const cavb200_bussi_args* bussi, void* stream, bool wrap,
+                            bool bath = false)
     {
     if (!h)
         return (int)cudaErrorInvalidValue;
     if (N == 0)
         return 0;
     MdArgs a;
-    if (const int rc = md_args(a, h, pos, vel, force_other, charge, image, N, Lx, Ly, Lz, L_typeid, params, group_first,
-                               n_group, bussi, wrap))
+    if (const int rc = md_args(a, h, pos, vel, force_other, charge, image, N, dt, Lx, Ly, Lz, L_typeid, params,
+                               group_first, n_group, bussi, wrap, bath, nullptr))
         return rc;
     const int grid = grid_for(h, N, 3, true); // one wave of 3 CTAs per SM (85-register budget)
     Final* fin_out = const_cast<Final*>(rank1_final(h));
     with_flags(
-        [&](auto WRAP, auto MASK)
+        [&](auto WRAP, auto MASK, auto BATH)
         {
-            k_md_one<WRAP, MASK><<<grid, 256, 0, (cudaStream_t)stream>>>((double4*)pos, (double4*)vel,
-                                                                        (const double4*)force_other, N, dt, a.b, h->scalars,
-                                                                        a.r, a.fnew, h->partials, h->counters + 4, fin_out,
-                                                                        a.w, a.mask);
+            if constexpr (!BATH || WRAP)
+                k_md_one<WRAP, MASK, BATH><<<grid, 256, 0, (cudaStream_t)stream>>>(
+                    (double4*)pos, (double4*)vel, (const double4*)force_other, N, dt, a.b, h->scalars, a.r, a.fnew,
+                    h->partials, h->counters + 4, fin_out, a.w, a.mask, a.bath);
         },
-        wrap, a.mask != nullptr);
+        wrap, a.mask != nullptr, bath);
     return launched(h);
     }
 
@@ -906,18 +992,31 @@ extern "C" int cavb200_md_step_one_wrap(cavb200_handle* h, double* pos, double* 
                             bussi, stream, true);
     }
 
+extern "C" int cavb200_md_step_one_wrap_bath(cavb200_handle* h, double* pos, double* vel, const double* force_other,
+                                             const double* charge, int32_t* image, uint32_t N, double dt, double Lx,
+                                             double Ly, double Lz, uint32_t L_typeid, const cavb200_params* params,
+                                             uint32_t group_first, uint32_t n_group, const cavb200_bussi_args* bussi,
+                                             void* stream)
+    {
+    return md_step_one_impl(h, pos, vel, force_other, charge, image, N, dt, Lx, Ly, Lz, L_typeid, params, group_first, n_group,
+                            bussi, stream, true, true);
+    }
+
 static int md_step_fused_impl(cavb200_handle* h, double* pos, double* vel, const double* force_other,
                               const double* charge, const int32_t* image, uint32_t N, double dt, double Lx,
                               double Ly, double Lz, uint32_t L_typeid, const cavb200_params* params,
-                              uint32_t group_first, uint32_t n_group, const cavb200_bussi_args* bussi, void* stream, bool wrap)
+                              uint32_t group_first, uint32_t n_group, const cavb200_bussi_args* bussi, void* stream, bool wrap,
+                              bool bath = false, const cavb200_langevin_args* draws = nullptr)
     {
     if (!h)
         return (int)cudaErrorInvalidValue;
     if (N == 0)
         return 0;
     MdArgs a;
-    if (const int rc = md_args(a, h, pos, vel, force_other, charge, image, N, Lx, Ly, Lz, L_typeid, params, group_first,
-                               n_group, bussi, wrap))
+    if (bath && !draws)
+        return (int)cudaErrorInvalidValue;
+    if (const int rc = md_args(a, h, pos, vel, force_other, charge, image, N, dt, Lx, Ly, Lz, L_typeid, params,
+                               group_first, n_group, bussi, wrap, bath, draws))
         return rc;
     if (!h->coop_supported)
         return (int)cudaErrorNotSupported;
@@ -926,9 +1025,14 @@ static int md_step_fused_impl(cavb200_handle* h, double* pos, double* vel, const
     // md_shape 1: two 384-thread CTAs per SM; otherwise one 768-thread CTA per SM (the folder CTA alone on its SM)
     const bool two = h->tune.md_shape == 1;
     const int threads = two ? 384 : 768, per_sm_want = two ? 2 : 1;
-    const void* kern;
-    with_flags([&](auto TWO, auto WRAP, auto MASK) { kern = (const void*)k_md_fused<TWO ? 384 : 768, 1, WRAP, MASK>; },
-               two, wrap, a.mask != nullptr);
+    const void* kern = nullptr;
+    with_flags(
+        [&](auto TWO, auto WRAP, auto MASK, auto BATH)
+        {
+            if constexpr (!BATH || WRAP)
+                kern = (const void*)k_md_fused<TWO ? 384 : 768, 1, WRAP, MASK, BATH>;
+        },
+        two, wrap, a.mask != nullptr, bath);
     int per_sm = 0;
     CAVB_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, 0));
     if (per_sm < 1)
@@ -950,7 +1054,7 @@ static int md_step_fused_impl(cavb200_handle* h, double* pos, double* vel, const
     Scalars* sca = h->scalars;
     unsigned long long* ctr = h->counters + 2;
     Final* fin_out = const_cast<Final*>(rank1_final(h));
-    void* args[] = {&p4, &v4, &fo4, &N, &dt, &a.b, &a.r, &a.fnew, &recsF, &recsB, &finals, &sca, &ctr, &fin_out, &a.w, &a.mask};
+    void* args[] = {&p4, &v4, &fo4, &N, &dt, &a.b, &a.r, &a.fnew, &recsF, &recsB, &finals, &sca, &ctr, &fin_out, &a.w, &a.mask, &a.bath};
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(threads);
@@ -990,6 +1094,16 @@ extern "C" int cavb200_md_step_fused_wrap(cavb200_handle* h, double* pos, double
     {
     return md_step_fused_impl(h, pos, vel, force_other, charge, image, N, dt, Lx, Ly, Lz, L_typeid, params, group_first,
                               n_group, bussi, stream, true);
+    }
+
+extern "C" int cavb200_md_step_fused_wrap_bath(cavb200_handle* h, double* pos, double* vel, const double* force_other,
+                                               const double* charge, int32_t* image, uint32_t N, double dt, double Lx,
+                                               double Ly, double Lz, uint32_t L_typeid, const cavb200_params* params,
+                                               uint32_t group_first, uint32_t n_group, const cavb200_bussi_args* bussi,
+                                               const cavb200_langevin_args* bath, void* stream)
+    {
+    return md_step_fused_impl(h, pos, vel, force_other, charge, image, N, dt, Lx, Ly, Lz, L_typeid, params, group_first,
+                              n_group, bussi, stream, true, true, bath);
     }
 
 extern "C" int cavb200_net_force_add_rank1(cavb200_handle* h, double* net_force, const double* charge, const double* pos,

@@ -480,7 +480,7 @@ class ParticleGroup
 //! reference's arithmetic given the draws is what gets pinned (SURVEY.md section 8c).
 struct RNGIdentifier
     {
-    enum Enum { BussiThermostat = 0x6a1, MTTKThermostat = 0x6a2 };
+    enum Enum { BussiThermostat = 0x6a1, MTTKThermostat = 0x6a2, TwoStepLangevin = 0x6a3 };
     };
 struct Seed
     {
@@ -530,6 +530,16 @@ template<class Real> class GammaDistribution
     Real operator()(RandomGenerator& rng) { return Real(rng.next()) * m_b; }
     private:
     Real m_alpha, m_b;
+    };
+
+template<class Real> class UniformDistribution
+    {
+    public:
+    UniformDistribution(Real a = 0, Real b = 1) : m_a(a), m_b(b) { }
+    //! the injected value is the variate itself
+    Real operator()(RandomGenerator& rng) { return Real(rng.next()); }
+    private:
+    Real m_a, m_b;
     };
 
 namespace md

@@ -83,6 +83,17 @@ typedef struct
     double gamma_draw;
     } cavb200_bussi_args;
 
+/* The cavity mode's own Langevin bath (HOOMD's TwoStepLangevin on the photon particle, type 'L'), the draws of ONE
+ * step two.  The bath force of the photon is bd_c = coeff r_c - gamma v_c with coeff = sqrt(6 gamma kT / dt), v the
+ * photon's velocity before its second half kick; the photon kicks with f = (f_other + F_L) + bd, and the first half kick
+ * of the next step uses the same bd (HOOMD keeps that sum as the acceleration).  See the *_bath entry points below. */
+typedef struct
+    {
+    double gamma; /* friction, >= 0 */
+    double kT;    /* bath temperature at this timestep, >= 0 */
+    double r[3];  /* three draws uniform in [-1, 1] */
+    } cavb200_langevin_args;
+
 /* ---- lifetime ------------------------------------------------------------------------------ */
 
 int cavb200_version(void);
@@ -264,6 +275,34 @@ int cavb200_md_step_fused_wrap(cavb200_handle* h, double* pos, double* vel, cons
                                int32_t* image, uint32_t N, double dt, double Lx, double Ly, double Lz, uint32_t L_typeid,
                                const cavb200_params* params, uint32_t group_first, uint32_t n_group,
                                const cavb200_bussi_args* bussi, void* stream);
+/* ... and with the cavity mode's Langevin bath (cavb200_langevin_args).  The handle keeps the photon's bath force bd[3]
+ * in a device slot: zero at cavb200_create, written by every step two that takes `bath`.  The bath acts on the photon of
+ * the last rank-1 result (Final.photon_local) and nowhere else; without a photon it does nothing.  A photon inside the
+ * thermostatted group still gets Bussi's alpha.  Each takes its sibling's arguments:
+ *   cavb200_nvt_step_two_rank1_bath      + `bath`: forms bd from the photon's velocity before the kick, kicks with it and
+ *                                        stores it in the slot
+ *   cavb200_nvt_step_one_rank1_wrap_bath the photon's kick adds the stored bd
+ *   cavb200_md_step_one_wrap_bath        the photon's kick adds the stored bd
+ *   cavb200_md_step_fused_wrap_bath      + `bath`: the draws of the DEFERRED step two (the previous step); bd is formed
+ *                                        once, used for both half kicks and stored
+ * cudaErrorInvalidValue for a NULL `bath`, gamma < 0, kT < 0 or dt <= 0. */
+int cavb200_nvt_step_two_rank1_bath(cavb200_handle* h, double* vel, const double* force_other, const double* charge,
+                                    const double* pos, uint32_t N, double dt, uint32_t L_typeid, double couplstr,
+                                    uint32_t group_first, uint32_t n_group, const cavb200_langevin_args* bath,
+                                    void* stream);
+int cavb200_nvt_step_one_rank1_wrap_bath(cavb200_handle* h, double* pos, double* vel, const double* force_other,
+                                         const double* charge, int32_t* image, uint32_t N, double dt, double Lx,
+                                         double Ly, double Lz, uint32_t L_typeid, double couplstr, uint32_t group_first,
+                                         uint32_t n_group, const cavb200_bussi_args* bussi, void* stream);
+int cavb200_md_step_one_wrap_bath(cavb200_handle* h, double* pos, double* vel, const double* force_other,
+                                  const double* charge, int32_t* image, uint32_t N, double dt, double Lx, double Ly,
+                                  double Lz, uint32_t L_typeid, const cavb200_params* params, uint32_t group_first,
+                                  uint32_t n_group, const cavb200_bussi_args* bussi, void* stream);
+int cavb200_md_step_fused_wrap_bath(cavb200_handle* h, double* pos, double* vel, const double* force_other,
+                                    const double* charge, int32_t* image, uint32_t N, double dt, double Lx, double Ly,
+                                    double Lz, uint32_t L_typeid, const cavb200_params* params, uint32_t group_first,
+                                    uint32_t n_group, const cavb200_bussi_args* bussi,
+                                    const cavb200_langevin_args* bath, void* stream);
 
 /* ---- index-list groups and particle sorts -------------------------------------------------------
  * HOOMD hands a group out as an index list, and its particle sorter permutes the particle arrays.

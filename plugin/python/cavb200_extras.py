@@ -40,6 +40,18 @@ def total_dipole(cavity_force):
     return _cpp(cavity_force).getDipole()
 
 
+def set_photon_bath(simulation, method, filter, kT, gamma):
+    """Give the cavity mode (the one particle of type 'L' that `filter` selects) its own Langevin bath inside the fused
+    method of make_fused_method ("rank1" or "one_launch" mode): HOOMD's TwoStepLangevin on the photon, in the method's
+    own launches.  Use it INSTEAD of hoomd.md.methods.Langevin(filter=photon), which would integrate the photon a second
+    time.  kT: a number or a hoomd.variant.Variant; gamma >= 0 (the reference's run: tau = 5 ps, gamma = 1 / tau).  The
+    photon must not be in the method's thermostatted group.  method.clearPhotonBath() removes the bath."""
+    if isinstance(kT, (int, float)):
+        import hoomd
+        kT = hoomd.variant.Constant(float(kT))
+    method.setPhotonBath(simulation.state._get_group(filter), kT, float(gamma))
+
+
 def make_fused_method(simulation, filter, bussi, cavity_force, mode="rank1"):
     """The fused integration method (plugin/src/TwoStepConstantVolumeCavity.h) as a C++ object, built from attached
     wrapper objects: thermostat folded into the kicks, cavity force rank-1 ("rank1"), or one launch per MD step

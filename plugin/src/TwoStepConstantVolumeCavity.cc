@@ -13,7 +13,8 @@ TwoStepConstantVolumeCavity::TwoStepConstantVolumeCavity(std::shared_ptr<SystemD
                                                          const std::string& mode)
     : IntegrationMethodTwoStep(sysdef, group), m_thermostat(thermostat), m_source(nullptr), m_cavity(cavity),
       m_handle(nullptr), m_started(false), m_pending(false), m_index_list(false), m_group_stale(true), m_use_mask(false),
-      m_first(0), m_group_n(0), m_group_N(0), m_photon_stale(false)
+      m_first(0), m_group_n(0), m_group_N(0), m_photon_stale(false), m_bath_gamma(0), m_bath_primed(false),
+      m_pending_bath(false), m_pending_args()
     {
     if (!m_exec_conf->isCUDAEnabled())
         throw std::runtime_error("TwoStepConstantVolumeCavity requires a GPU execution configuration (no CPU fallback)");
@@ -158,6 +159,61 @@ void TwoStepConstantVolumeCavity::reindexPhoton(uint32_t L_typeid)
     m_photon_stale = false;
     }
 
+void TwoStepConstantVolumeCavity::setPhotonBath(std::shared_ptr<ParticleGroup> photon_group, std::shared_ptr<Variant> kT,
+                                                Scalar gamma)
+    {
+    if (m_mode == STORED)
+        throw std::invalid_argument("TwoStepConstantVolumeCavity: the photon bath needs the 'rank1' or 'one_launch' mode "
+                                    "(the stored mode's handle does not know the photon)");
+    if (!photon_group || !kT)
+        throw std::invalid_argument("TwoStepConstantVolumeCavity: the photon bath needs a group and a kT variant");
+    if (!(gamma >= 0))
+        throw std::invalid_argument("TwoStepConstantVolumeCavity: the photon bath needs gamma >= 0");
+    if (!((*kT)(0) >= 0))
+        throw std::invalid_argument("TwoStepConstantVolumeCavity: the photon bath needs kT >= 0");
+    if (photon_group->getNumMembers() != 1)
+        throw std::invalid_argument("TwoStepConstantVolumeCavity: the photon bath group must hold exactly one particle");
+    const unsigned int tag = photon_group->getMemberTag(0);
+        {
+        ArrayHandle<Scalar4> h_pos(m_pdata->getPositions(), access_location::host, access_mode::read);
+        if (__scalar_as_int(h_pos.data[m_pdata->getRTag(tag)].w) != (int)photonTypeId())
+            throw std::invalid_argument("TwoStepConstantVolumeCavity: the photon bath group's particle must have type 'L'");
+        }
+    for (unsigned int j = 0; j < m_group->getNumMembers(); j++)
+        if (m_group->getMemberTag(j) == tag)
+            throw std::invalid_argument("TwoStepConstantVolumeCavity: the photon is in the thermostatted group; the photon "
+                                        "bath needs it outside (it would get both baths)");
+    m_bath_group = photon_group;
+    m_bath_kT = kT;
+    m_bath_gamma = gamma;
+    m_bath_primed = false; // bd = 0 until the first step two with this bath (HOOMD: the first accelerations are F / m)
+    }
+
+void TwoStepConstantVolumeCavity::clearPhotonBath()
+    {
+    m_bath_group.reset();
+    m_bath_kT.reset();
+    m_bath_primed = false;
+    }
+
+cavb200_langevin_args TwoStepConstantVolumeCavity::drawBath(uint64_t timestep)
+    {
+    // HOOMD's TwoStepLangevin [HOOMD-upstream: restated]: three uniform draws in [-1, 1] per particle and step, the
+    // stream keyed by the timestep, the simulation seed and the particle's tag (a sort does not change them)
+    cavb200_langevin_args a = {};
+    a.gamma = m_bath_gamma;
+    a.kT = (*m_bath_kT)(timestep);
+    if (!(a.kT >= 0))
+        throw std::runtime_error("TwoStepConstantVolumeCavity: the photon bath's kT is negative at this timestep");
+    RandomGenerator rng(Seed(RNGIdentifier::TwoStepLangevin, timestep, m_sysdef->getSeed()),
+                        Counter(m_bath_group->getMemberTag(0)));
+    UniformDistribution<Scalar> uniform(Scalar(-1), Scalar(1));
+    a.r[0] = uniform(rng);
+    a.r[1] = uniform(rng);
+    a.r[2] = uniform(rng);
+    return a;
+    }
+
 void TwoStepConstantVolumeCavity::integrateStepOne(uint64_t timestep)
     {
     const unsigned int N = m_pdata->getN();
@@ -204,20 +260,31 @@ void TwoStepConstantVolumeCavity::integrateStepOne(uint64_t timestep)
               "cavb200_nvt_step_one_wrap");
         break;
     case RANK1:
-        check(cavb200_nvt_step_one_rank1_wrap(m_handle, pos, vel, net, d_charge.data, image, N, m_deltaT, L.x, L.y, L.z,
-                                              L_typeid, m_cavity->params().couplstr, first, n, bussi, nullptr),
+        // with the bath, the photon's kick adds the bd the last step two stored
+        check((m_bath_group && m_bath_primed ? cavb200_nvt_step_one_rank1_wrap_bath : cavb200_nvt_step_one_rank1_wrap)(
+                  m_handle, pos, vel, net, d_charge.data, image, N, m_deltaT, L.x, L.y, L.z, L_typeid,
+                  m_cavity->params().couplstr, first, n, bussi, nullptr),
               "cavb200_nvt_step_one_rank1_wrap");
         break;
     case ONE_LAUNCH:
-        if (m_pending)
+        if (m_pending && m_pending_bath)
+            {
+            check(cavb200_md_step_fused_wrap_bath(m_handle, pos, vel, net, d_charge.data, image, N, m_deltaT, L.x, L.y, L.z,
+                                                  L_typeid, &m_cavity->params(), first, n, bussi, &m_pending_args, nullptr),
+                  "cavb200_md_step_fused_wrap_bath");
+            m_bath_primed = true;
+            }
+        else if (m_pending)
             check(cavb200_md_step_fused_wrap(m_handle, pos, vel, net, d_charge.data, image, N, m_deltaT, L.x, L.y, L.z,
                                              L_typeid, &m_cavity->params(), first, n, bussi, nullptr),
                   "cavb200_md_step_fused_wrap");
         else
-            check(cavb200_md_step_one_wrap(m_handle, pos, vel, net, d_charge.data, image, N, m_deltaT, L.x, L.y, L.z, L_typeid,
-                                           &m_cavity->params(), first, n, bussi, nullptr),
+            check((m_bath_group && m_bath_primed ? cavb200_md_step_one_wrap_bath : cavb200_md_step_one_wrap)(
+                      m_handle, pos, vel, net, d_charge.data, image, N, m_deltaT, L.x, L.y, L.z, L_typeid,
+                      &m_cavity->params(), first, n, bussi, nullptr),
                   "cavb200_md_step_one_wrap");
         m_pending = false;
+        m_pending_bath = false;
         m_cavity->integratorHasReduced(); // the dipole of the new positions is on the device: compute() has nothing to do
         break;
         }
@@ -225,13 +292,17 @@ void TwoStepConstantVolumeCavity::integrateStepOne(uint64_t timestep)
 
 void TwoStepConstantVolumeCavity::integrateStepTwo(uint64_t timestep)
     {
-    (void)timestep;
     const unsigned int N = m_pdata->getN();
     if (N == 0)
         return;
+    cavb200_langevin_args bath = {};
+    if (m_bath_group && m_mode != STORED)
+        bath = drawBath(timestep);
     if (m_mode == ONE_LAUNCH)
         {
         m_pending = true; // rides on the next step one (or flush())
+        m_pending_bath = (bool)m_bath_group;
+        m_pending_args = bath;
         return;
         }
     unsigned int first = 0, n = 0;
@@ -249,6 +320,14 @@ void TwoStepConstantVolumeCavity::integrateStepTwo(uint64_t timestep)
         }
     ArrayHandle<Scalar4> d_pos(m_pdata->getPositions(), access_location::device, access_mode::read);
     ArrayHandle<Scalar> d_charge(m_pdata->getCharges(), access_location::device, access_mode::read);
+    if (m_bath_group)
+        {
+        check(cavb200_nvt_step_two_rank1_bath(m_handle, vel, net, d_charge.data, reinterpret_cast<const double*>(d_pos.data),
+                                              N, m_deltaT, L_typeid, m_cavity->params().couplstr, first, n, &bath, nullptr),
+              "cavb200_nvt_step_two_rank1_bath");
+        m_bath_primed = true;
+        return;
+        }
     check(cavb200_nvt_step_two_rank1(m_handle, vel, net, d_charge.data, reinterpret_cast<const double*>(d_pos.data), N,
                                      m_deltaT, L_typeid, m_cavity->params().couplstr, first, n, nullptr),
           "cavb200_nvt_step_two_rank1");
@@ -267,11 +346,23 @@ void TwoStepConstantVolumeCavity::flush()
     ArrayHandle<Scalar4> d_net(m_pdata->getNetForce(), access_location::device, access_mode::read);
     ArrayHandle<Scalar4> d_pos(m_pdata->getPositions(), access_location::device, access_mode::read);
     ArrayHandle<Scalar> d_charge(m_pdata->getCharges(), access_location::device, access_mode::read);
-    check(cavb200_nvt_step_two_rank1(m_handle, reinterpret_cast<double*>(d_vel.data), reinterpret_cast<const double*>(d_net.data),
-                                     d_charge.data, reinterpret_cast<const double*>(d_pos.data), N, m_deltaT, L_typeid,
-                                     m_cavity->params().couplstr, first, n, nullptr),
-          "cavb200_nvt_step_two_rank1");
+    if (m_pending_bath)
+        {
+        check(cavb200_nvt_step_two_rank1_bath(m_handle, reinterpret_cast<double*>(d_vel.data),
+                                              reinterpret_cast<const double*>(d_net.data), d_charge.data,
+                                              reinterpret_cast<const double*>(d_pos.data), N, m_deltaT, L_typeid,
+                                              m_cavity->params().couplstr, first, n, &m_pending_args, nullptr),
+              "cavb200_nvt_step_two_rank1_bath");
+        m_bath_primed = true;
+        }
+    else
+        check(cavb200_nvt_step_two_rank1(m_handle, reinterpret_cast<double*>(d_vel.data),
+                                         reinterpret_cast<const double*>(d_net.data), d_charge.data,
+                                         reinterpret_cast<const double*>(d_pos.data), N, m_deltaT, L_typeid,
+                                         m_cavity->params().couplstr, first, n, nullptr),
+              "cavb200_nvt_step_two_rank1");
     m_pending = false;
+    m_pending_bath = false;
     // the velocities are now complete, but the next step one must not redo this half kick: restart from md_step_one
     }
 
@@ -289,7 +380,11 @@ void export_TwoStepConstantVolumeCavity(pybind11::module& m)
         .def_property_readonly("mode", &TwoStepConstantVolumeCavity::getMode)
         .def_property("index_list_group", &TwoStepConstantVolumeCavity::getIndexListGroup,
                       &TwoStepConstantVolumeCavity::setIndexListGroup)
-        .def("getLaunchCount", &TwoStepConstantVolumeCavity::getLaunchCount);
+        .def("getLaunchCount", &TwoStepConstantVolumeCavity::getLaunchCount)
+        .def("setPhotonBath", &TwoStepConstantVolumeCavity::setPhotonBath, py::arg("photon_group"), py::arg("kT"),
+             py::arg("gamma"))
+        .def("clearPhotonBath", &TwoStepConstantVolumeCavity::clearPhotonBath)
+        .def_property_readonly("photon_bath", &TwoStepConstantVolumeCavity::hasPhotonBath);
     }
     } // namespace detail
     } // namespace hoomd::md

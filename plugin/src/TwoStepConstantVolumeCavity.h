@@ -24,14 +24,23 @@
 // handle's bit mask (cavb200_group_set, CAVB200_GROUP_MASK), rebuilt when HOOMD's particle sorter has reordered the
 // particles or the group / particle count changed.  In either case a sort (getParticleSortSignal) also moves the photon
 // index of the last rank-1 result (cavb200_rank1_reindex) in the rank1 and one_launch modes, before the next launch.
+// Photon bath (setPhotonBath, rank1 and one_launch modes): the cavity mode gets its own Langevin bath, HOOMD's
+// TwoStepLangevin on the one particle of type 'L' [HOOMD-upstream: restated], in the same launches (the *_bath entry
+// points of include/cavb200.h).  integrateStepTwo draws r with RandomGenerator(Seed(RNGIdentifier::TwoStepLangevin, t,
+// seed), Counter(photon tag)) and evaluates kT(t); the photon kicks with f + bd, bd = coeff r - gamma v.  This replaces
+// hoomd.md.methods.Langevin(filter=photon) next to the method, which would integrate the photon twice.
 // Restrictions (checked, stated in INTEGRATION.md): every particle of the system is integrated by this method; point
-// particles only; single rank; with the sorter on, one particle of type 'L' in the rank-1 modes.
+// particles only; single rank; with the sorter on, one particle of type 'L' in the rank-1 modes; the photon bath acts on
+// a group of exactly that one particle, outside the thermostatted group, not in the stored mode.
 #ifndef CAVB200_TWO_STEP_CONSTANT_VOLUME_CAVITY_H
 #define CAVB200_TWO_STEP_CONSTANT_VOLUME_CAVITY_H
 
 #include "CavbHooks.h"
 #include "CavityForceComputeGPU.h"
 
+#include <hoomd/RNGIdentifiers.h>
+#include <hoomd/RandomNumbers.h>
+#include <hoomd/Variant.h>
 #include <hoomd/md/IntegrationMethodTwoStep.h>
 #include <hoomd/md/Thermostat.h>
 
@@ -59,6 +68,10 @@ class PYBIND11_EXPORT TwoStepConstantVolumeCavity : public IntegrationMethodTwoS
     void setIndexListGroup(bool on);
     //! HOOMD's particle sort signal: the mask and the photon index are rebuilt before the next launch
     void slotParticleSort();
+    //! the cavity mode's Langevin bath on photon_group (one particle of type 'L', not thermostatted): kT(t), gamma >= 0
+    void setPhotonBath(std::shared_ptr<ParticleGroup> photon_group, std::shared_ptr<Variant> kT, Scalar gamma);
+    void clearPhotonBath();
+    bool hasPhotonBath() const { return (bool)m_bath_group; }
 
     private:
     void window(unsigned int& first, unsigned int& n);
@@ -80,6 +93,13 @@ class PYBIND11_EXPORT TwoStepConstantVolumeCavity : public IntegrationMethodTwoS
     unsigned int m_first;  //!< index_list_group: first index of a contiguous group
     unsigned int m_group_n, m_group_N; //!< members and particle count the window / mask was built for
     bool m_photon_stale;   //!< particles were sorted since the last rank-1 result was formed
+    std::shared_ptr<ParticleGroup> m_bath_group; //!< photon bath: its group (nullptr: no bath)
+    std::shared_ptr<Variant> m_bath_kT;
+    Scalar m_bath_gamma;
+    bool m_bath_primed;    //!< photon bath: a step two with the bath has stored bd in the handle's slot
+    bool m_pending_bath;   //!< one_launch: the outstanding second half kick takes m_pending_args
+    cavb200_langevin_args m_pending_args;
+    cavb200_langevin_args drawBath(uint64_t timestep);
     };
 
 namespace detail
