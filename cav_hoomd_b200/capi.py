@@ -117,6 +117,9 @@ _SIGNATURES = {
     "cavb200_rhok": (C.c_int, [_vp, _vp, _u32, _u64, _u32, _u32, _vp, _u32, _vp, _vp]),
     "cavb200_rhok_f32": (C.c_int, [_vp, _vp, _u64, _u32, _u32, _vp, _u32, _vp, _vp]),
     "cavb200_fkt": (C.c_int, [_vp, _vp, _u32, _u32, _u32, _u32, _vp, _vp]),
+    "cavb200_fkt_track_open": (C.c_int, [_vp, _dp, _u32, _u32, _u32, _u32]),
+    "cavb200_fkt_track_step": (C.c_int, [_vp, _vp, _u32, _u64, _u32, _vp]),
+    "cavb200_fkt_track_read": (C.c_int, [_vp, _dp, _u32, C.POINTER(_u32), C.POINTER(_u64), _vp]),
     "cavb200_shard_nccl_unique_id": (C.c_int, [_vp]),
     "cavb200_shard_init_nccl": (C.c_int, [_vp, _vp, C.c_int, C.c_int]),
     "cavb200_shard_mailbox_export": (C.c_int, [_vp, _vp]),
@@ -604,6 +607,28 @@ class Handle:
 
     def fkt(self, rho, T, K, n_origins, n_lags, out, stream=None):
         check(self.lib.cavb200_fkt(self.h, _ptr(rho), T, K, n_origins, n_lags, _ptr(out), stream), "cavb200_fkt")
+
+    # -- F(k,t) tracker without snapshots -----------------------------------------------------------
+    FKT_RECORD, FKT_ADD_REFERENCE = 1, 2  # CAVB200_FKT_RECORD, CAVB200_FKT_ADD_REFERENCE
+
+    def fkt_track_open(self, kvec, max_references: int, capacity: int, N: int):
+        """kvec: host wave vectors [K, 3].  Blocking; drops every stored reference and empties the ring."""
+        k = np.ascontiguousarray(kvec, dtype=np.float64).reshape(-1, 3)
+        check(self.lib.cavb200_fkt_track_open(self.h, k.ctypes.data_as(_dp), k.shape[0], max_references, capacity, N),
+              "cavb200_fkt_track_open")
+        self._fkt_words = 2 + int(max_references) + 2 * k.shape[0]
+
+    def fkt_track_step(self, pos, N: int, timestep: int, flags: int, stream=None):
+        check(self.lib.cavb200_fkt_track_step(self.h, _ptr(pos), N, timestep, flags, stream), "cavb200_fkt_track_step")
+
+    def fkt_track_read(self, max_records: int, stream=None):
+        """-> (records float64[n, 2 + max_references + 2K] oldest first, total appended since open)"""
+        words = getattr(self, "_fkt_words", 1)
+        out = np.zeros((max(max_records, 1), words), dtype=np.float64)
+        n, total = C.c_uint32(0), C.c_uint64(0)
+        check(self.lib.cavb200_fkt_track_read(self.h, out.ctypes.data_as(_dp), max_records, C.byref(n), C.byref(total),
+                                              stream), "cavb200_fkt_track_read")
+        return out[:n.value], int(total.value)
 
     # -- sharded ---------------------------------------------------------------------------------
     def nccl_unique_id(self) -> bytes:

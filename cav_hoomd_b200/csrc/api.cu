@@ -204,6 +204,7 @@ int cavb200_destroy(cavb200_handle* h)
     cavb_shard_release(h);
     cavb_host_release(h);
     cavb_track_release(h);
+    cavb_fkt_track_release(h);
     cudaFree(h->partials);
     cudaFree(h->scalars);
     cudaFree(h->counters);

@@ -149,6 +149,12 @@ struct cavb200_handle
     double* rhok_partials;
     uint64_t rhok_partials_bytes;
     void* rhok_table; // device, (cos, sin)(2 pi e / 512) as double2 (rhok.cu)
+    // F(k,t) tracker (rhok.cu, cavb200_fkt_track_*): one allocation holding the wave vectors [3K] | rho slot [2K] |
+    // stored references [max_refs][2K] | ring [capacity][2 + max_refs + 2K] | record counter; the reference count is
+    // kept here on the host
+    double* fkt_track;
+    uint32_t fkt_K, fkt_max_refs, fkt_n_refs;
+    uint64_t fkt_capacity;
     // thermostatted group as a bit mask (cavb200_group_set), used by the window entry points with CAVB200_GROUP_MASK
     uint32_t* group_mask;             // device, ceil(N / 32) words
     uint64_t group_mask_words;        // allocated words
@@ -351,6 +357,7 @@ __device__ __forceinline__ double shfl_xor_d(double v, int m) { return __shfl_xo
 void cavb_shard_release(cavb200_handle* h);
 void cavb_host_release(cavb200_handle* h);
 void cavb_track_release(cavb200_handle* h);
+void cavb_fkt_track_release(cavb200_handle* h);
 
 // launch helpers implemented in the .cu files
 namespace cavb

@@ -381,7 +381,20 @@ __global__ void k_rhok_fold(const double* __restrict__ part, uint32_t P, uint32_
         }
     }
 
-// F[o][l] = mean_k Re(rho[o][k] conj(rho[o+l][k]))  (analysis.py:361: np.mean(np.real(f0 * np.conj(ft))))
+// mean_k Re(a_k conj(b_k)) of two fields of K {re, im} pairs, k ascending (analysis.py:361:
+// np.mean(np.real(f0 * np.conj(ft)))).  The one loop of k_fkt and k_fkt_track, so that both give the same bits.
+__device__ __forceinline__ double fkt_pair(const double* a, const double* b, uint32_t K)
+    {
+    double acc = 0.0;
+    for (uint32_t k = 0; k < K; k++)
+        {
+        // Re((ar + i ai)(br - i bi)) = ar br + ai bi
+        acc += a[2 * k] * b[2 * k] + a[2 * k + 1] * b[2 * k + 1];
+        }
+    return acc / (double)K;
+    }
+
+// F[o][l] = mean_k Re(rho[o][k] conj(rho[o+l][k]))
 __global__ void k_fkt(const double* __restrict__ rho, uint32_t T, uint32_t K, uint32_t n_origins, uint32_t n_lags,
                       double* __restrict__ out)
     {
@@ -394,15 +407,40 @@ __global__ void k_fkt(const double* __restrict__ rho, uint32_t T, uint32_t K, ui
         out[e] = __longlong_as_double(0x7ff8000000000000ll);
         return;
         }
-    const double* a = rho + o * K * 2;
-    const double* b = rho + (o + l) * K * 2;
-    double acc = 0.0;
-    for (uint32_t k = 0; k < K; k++)
+    out[e] = fkt_pair(rho + o * K * 2, rho + (o + l) * K * 2, K);
+    }
+
+// F(k,t) tracker step (cavb200_fkt_track_step): after k_rhok (and k_rhok_fold) have written this frame's rho into the
+// slot, one CTA appends the record {timestep, n_refs, F of every stored reference against rho (NaN past n_refs), rho}
+// to the ring (RECORD) and/or copies rho into reference slot n_refs (ADD_REFERENCE).  Thread j < max_refs forms F of
+// reference j with the loop k_fkt uses, so a record is bit-identical to cavb200_fkt on (reference j, this frame).
+__global__ void k_fkt_track(const double* __restrict__ rho, double* __restrict__ refs, uint32_t K, uint32_t max_refs,
+                            uint32_t n_refs, uint32_t flags, double timestep, double* __restrict__ ring,
+                            unsigned long long* __restrict__ count, unsigned long long capacity)
+    {
+    const uint32_t tid = threadIdx.x;
+    pdl_wait(); // rho is written by the launch before this one
+    pdl_launch_dependents();
+    if (flags & CAVB200_FKT_RECORD)
         {
-        // Re((ar + i ai)(br - i bi)) = ar br + ai bi
-        acc += a[2 * k] * b[2 * k] + a[2 * k + 1] * b[2 * k + 1];
+        const unsigned long long n = *count;
+        double* r = ring + (n % capacity) * (2ull + max_refs + 2ull * K);
+        if (tid == 0)
+            {
+            r[0] = timestep;
+            r[1] = (double)n_refs;
+            }
+        for (uint32_t j = tid; j < max_refs; j += blockDim.x)
+            r[2 + j] = j < n_refs ? fkt_pair(refs + 2ull * K * j, rho, K) : __longlong_as_double(0x7ff8000000000000ll);
+        for (uint32_t e = tid; e < 2 * K; e += blockDim.x)
+            r[2 + max_refs + e] = rho[e];
+        __syncthreads(); // every thread has read the counter
+        if (tid == 0)
+            *count = n + 1;
         }
-    out[e] = acc / (double)K;
+    if (flags & CAVB200_FKT_ADD_REFERENCE)
+        for (uint32_t e = tid; e < 2 * K; e += blockDim.x)
+            refs[2ull * K * n_refs + e] = rho[e];
     }
     } // namespace cavb
 
@@ -462,6 +500,45 @@ static uint32_t rhok_slices(uint32_t tiles, uint32_t T, uint32_t slots)
     return best;
     }
 
+// First use on a handle: the 8 KB table (a blocking copy from pageable memory, like the workspace growth in rhok_launch)
+// and the kernels' shared-memory limit.
+static int rhok_table_init(cavb200_handle* h)
+    {
+    if (h->rhok_table)
+        return 0;
+    double2 host_tab[RHOK_TAB];
+    rhok_table_host(host_tab);
+    CAVB_CHECK(cudaMalloc((void**)&h->rhok_table, sizeof(host_tab)));
+    CAVB_CHECK(cudaMemcpy(h->rhok_table, host_tab, sizeof(host_tab), cudaMemcpyHostToDevice));
+    const int smem_max = (int)(sizeof(double2) * RHOK_TAB * RHOK_REP + sizeof(double4) * 2 * RHOK_TILE);
+    CAVB_CHECK(cudaFuncSetAttribute(k_rhok<RHOK_KB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+    CAVB_CHECK(cudaFuncSetAttribute(k_rhok<RHOK_KB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+    return 0;
+    }
+
+// Everything rhok_launch would set up on first use for one frame (T = 1) of at most N particles and K wave vectors:
+// the table and a slice workspace no such call outgrows.  rhok_slices is not monotonic in the tile count, so the
+// workspace is sized for its upper limit min(tiles, RHOK_GRID_PER_SM * slots), which covers every N' <= N.  Blocking.
+static int rhok_prime(cavb200_handle* h, uint32_t N, uint32_t K)
+    {
+    if (const int err = rhok_table_init(h))
+        return err;
+    const uint64_t tiles = ((uint64_t)N + RHOK_TILE - 1) / RHOK_TILE;
+    const uint64_t pmax = (uint64_t)RHOK_GRID_PER_SM * 2u * (uint64_t)h->num_sms;
+    const uint64_t P = tiles < pmax ? tiles : pmax;
+    const uint64_t need = P > 1 ? sizeof(double) * 2ull * K * P : 0;
+    if (h->rhok_partials_bytes < need)
+        {
+        CAVB_CHECK(cudaDeviceSynchronize());
+        cudaFree(h->rhok_partials);
+        h->rhok_partials = nullptr;
+        h->rhok_partials_bytes = 0;
+        CAVB_CHECK(cudaMalloc((void**)&h->rhok_partials, need));
+        h->rhok_partials_bytes = need;
+        }
+    return 0;
+    }
+
 static int rhok_launch(cavb200_handle* h, const double* pos, uint32_t stride, uint64_t frame_stride, uint32_t N,
                        uint32_t T, const double* kvec, uint32_t K, double* rho, void* stream)
     {
@@ -481,17 +558,8 @@ static int rhok_launch(cavb200_handle* h, const double* pos, uint32_t stride, ui
         CAVB_CHECK(cudaMemsetAsync(rho, 0, sizeof(double) * 2ull * K * T, s));
         return 0;
         }
-    if (!h->rhok_table)
-        {
-        // first call on this handle: the 8 KB table (a blocking copy from pageable memory, like the workspace growth below)
-        double2 host_tab[RHOK_TAB];
-        rhok_table_host(host_tab);
-        CAVB_CHECK(cudaMalloc((void**)&h->rhok_table, sizeof(host_tab)));
-        CAVB_CHECK(cudaMemcpy(h->rhok_table, host_tab, sizeof(host_tab), cudaMemcpyHostToDevice));
-        const int smem_max = (int)(sizeof(double2) * RHOK_TAB * RHOK_REP + sizeof(double4) * 2 * RHOK_TILE);
-        CAVB_CHECK(cudaFuncSetAttribute(k_rhok<RHOK_KB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-        CAVB_CHECK(cudaFuncSetAttribute(k_rhok<RHOK_KB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-        }
+    if (const int err = rhok_table_init(h))
+        return err;
     // two CTAs of 256 threads per SM: the 64 KB table of each leaves no room for four of 128 (which were worth 1-2 % when
     // the table was four entries: a CTA staging its next tile idled a quarter of the SM's warps instead of half)
     const int threads = (h->tune.rhok_threads >= 128 && h->tune.rhok_threads <= RHOK_CTA && h->tune.rhok_threads % 128 == 0)
@@ -606,5 +674,124 @@ extern "C" int cavb200_fkt(cavb200_handle* h, const double* rho, uint32_t T, uin
     k_fkt<<<(unsigned int)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(rho, T, K, n_origins, n_lags, out);
     CAVB_CHECK(cudaGetLastError());
     h->launches += 1;
+    return 0;
+    }
+
+// ---- F(k,t) tracker: rho(t) and its correlation with every stored reference, on the device, each step ----------------
+static uint64_t fkt_words(const cavb200_handle* h) { return 2ull + h->fkt_max_refs + 2ull * h->fkt_K; }
+static double* fkt_kvec(cavb200_handle* h) { return h->fkt_track; }
+static double* fkt_rho(cavb200_handle* h) { return h->fkt_track + 3ull * h->fkt_K; }
+static double* fkt_refs(cavb200_handle* h) { return fkt_rho(h) + 2ull * h->fkt_K; }
+static double* fkt_ring(cavb200_handle* h) { return fkt_refs(h) + 2ull * h->fkt_K * h->fkt_max_refs; }
+static unsigned long long* fkt_counter(cavb200_handle* h)
+    {
+    return reinterpret_cast<unsigned long long*>(fkt_ring(h) + h->fkt_capacity * fkt_words(h));
+    }
+
+void cavb_fkt_track_release(cavb200_handle* h)
+    {
+    cudaFree(h->fkt_track);
+    h->fkt_track = nullptr;
+    h->fkt_K = h->fkt_max_refs = h->fkt_n_refs = 0;
+    h->fkt_capacity = 0;
+    }
+
+extern "C" int cavb200_fkt_track_open(cavb200_handle* h, const double* kvec_host, uint32_t K, uint32_t max_references,
+                                      uint32_t capacity, uint32_t N)
+    {
+    if (!h || !kvec_host || K == 0 || max_references == 0 || max_references > 1024 || capacity == 0)
+        return (int)cudaErrorInvalidValue;
+    CAVB_CHECK(cudaSetDevice(h->device));
+    cavb_fkt_track_release(h);
+    const uint64_t words = 2ull + max_references + 2ull * K;
+    const size_t bytes = sizeof(double) * (5ull * K + 2ull * K * max_references + (uint64_t)capacity * words) +
+                         sizeof(unsigned long long);
+    double* buf = nullptr;
+    CAVB_CHECK(cudaMalloc((void**)&buf, bytes));
+    h->fkt_track = buf;
+    h->fkt_K = K;
+    h->fkt_max_refs = max_references;
+    h->fkt_capacity = capacity;
+    int err = (int)cudaMemset(buf, 0, bytes);
+    if (!err)
+        err = (int)cudaMemcpy(fkt_kvec(h), kvec_host, sizeof(double) * 3ull * K, cudaMemcpyHostToDevice);
+    // the table, the kernels' attributes and the slice workspace now, so that a step never synchronises
+    if (!err)
+        err = rhok_prime(h, N, K);
+    if (err)
+        cavb_fkt_track_release(h);
+    return err;
+    }
+
+extern "C" int cavb200_fkt_track_step(cavb200_handle* h, const double* pos, uint32_t N, uint64_t timestep, uint32_t flags,
+                                      void* stream)
+    {
+    if (!h || !h->fkt_track || flags == 0 || (flags & ~(CAVB200_FKT_RECORD | CAVB200_FKT_ADD_REFERENCE)))
+        return (int)cudaErrorInvalidValue;
+    if ((flags & CAVB200_FKT_ADD_REFERENCE) && h->fkt_n_refs >= h->fkt_max_refs)
+        return (int)cudaErrorInvalidValue;
+    const uint32_t K = h->fkt_K;
+    // rho(t) into the slot: the cavb200_rhok launch for one Scalar4 frame (its checks: NULL pos with N > 0, alignment)
+    const int err = rhok_launch(h, pos, 4, 4ull * N, N, 1, fkt_kvec(h), K, fkt_rho(h), stream);
+    if (err)
+        return err;
+    cudaLaunchAttribute pdl_attr;
+    pdl_attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    pdl_attr.val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    // one thread per reference (at most 1024), and at least 256 for the copies of rho
+    const uint32_t threads = h->fkt_max_refs <= 256 ? 256u : (h->fkt_max_refs + 31u) / 32u * 32u;
+    cfg.gridDim = dim3(1);
+    cfg.blockDim = dim3(threads);
+    cfg.stream = (cudaStream_t)stream;
+    cfg.attrs = &pdl_attr;
+    cfg.numAttrs = h->tune.pdl ? 1 : 0;
+    const double* rho = fkt_rho(h);
+    double* refs = fkt_refs(h);
+    uint32_t max_refs = h->fkt_max_refs, n_refs = h->fkt_n_refs;
+    double ts = (double)timestep;
+    double* ring = fkt_ring(h);
+    unsigned long long* count = fkt_counter(h);
+    unsigned long long cap = h->fkt_capacity;
+    void* args[] = {(void*)&rho, (void*)&refs, (void*)&K,  (void*)&max_refs, (void*)&n_refs,
+                    (void*)&flags, (void*)&ts, (void*)&ring, (void*)&count,    (void*)&cap};
+    CAVB_CHECK(cudaLaunchKernelExC(&cfg, (const void*)k_fkt_track, args));
+    h->launches += 1;
+    if (flags & CAVB200_FKT_ADD_REFERENCE)
+        h->fkt_n_refs += 1;
+    return 0;
+    }
+
+extern "C" int cavb200_fkt_track_read(cavb200_handle* h, double* out, uint32_t max_records, uint32_t* n_out,
+                                      uint64_t* total, void* stream)
+    {
+    if (!h || !h->fkt_track || (!out && max_records) || !n_out)
+        return (int)cudaErrorInvalidValue;
+    cudaStream_t s = (cudaStream_t)stream;
+    unsigned long long cnt = 0;
+    CAVB_CHECK(cudaMemcpyAsync(&cnt, fkt_counter(h), sizeof(cnt), cudaMemcpyDeviceToHost, s));
+    CAVB_CHECK(cudaStreamSynchronize(s));
+    const unsigned long long cap = h->fkt_capacity;
+    const uint64_t words = fkt_words(h);
+    unsigned long long have = cnt < cap ? cnt : cap; // records still in the ring
+    if (have > max_records)
+        have = max_records;
+    // the newest `have` records, oldest first; the ring wraps at most once inside that span
+    const unsigned long long first = cnt - have;
+    unsigned long long done = 0;
+    while (done < have)
+        {
+        const unsigned long long at = (first + done) % cap;
+        unsigned long long run = cap - at;
+        if (run > have - done)
+            run = have - done;
+        CAVB_CHECK(cudaMemcpyAsync(out + done * words, fkt_ring(h) + at * words, run * words * sizeof(double),
+                                   cudaMemcpyDeviceToHost, s));
+        done += run;
+        }
+    CAVB_CHECK(cudaStreamSynchronize(s));
+    *n_out = (uint32_t)have;
+    if (total)
+        *total = cnt;
     return 0;
     }

@@ -373,6 +373,36 @@ int cavb200_rhok_f32(cavb200_handle* h, const float* pos_xyz, uint64_t frame_str
 int cavb200_fkt(cavb200_handle* h, const double* rho, uint32_t T, uint32_t K, uint32_t n_origins,
                 uint32_t n_lags, double* out, void* stream);
 
+/* ---- F(k,t) tracker without snapshots -----------------------------------------------------------
+ * Replaces the per-step cpu_local_snapshot + K NumPy passes of FieldAutocorrelationTracker.act (reference
+ * src/cavitymd/analysis.py:260-418): each step computes rho(t) of the wrapped positions on the device (the
+ * cavb200_rhok launch, T = 1) and appends a record holding F of every stored reference against it, and rho(t)
+ * itself, to a ring in device memory; the host reads the ring once per output period.  Record layout
+ * (2 + max_references + 2K doubles):
+ *   [0] timestep   [1] number of references compared   [2 .. 2 + max_references) F of reference r =
+ *   mean_k Re(rho_r[k] conj(rho(t)[k])), bit-identical to cavb200_fkt on (reference r, this frame); NaN in the
+ *   unused slots   [2 + max_references ..) rho(t) as {re, im} pairs, bit-identical to cavb200_rhok (stride 4, T = 1).
+ *   cavb200_fkt_track_open   K wave vectors (host double[3K]), up to max_references (1..1024) stored fields, a ring of
+ *                            `capacity` records.  Blocking: uploads the wave vectors and sets up everything the
+ *                            density-field launch needs for frames of up to N particles, so that a step never
+ *                            synchronises (a larger N grows the workspace once, blocking, as cavb200_rhok does).
+ *                            Calling it again re-opens: the ring is emptied and every stored reference dropped.
+ *   cavb200_fkt_track_step   pos: Scalar4 positions of all N particles, photon included (32-byte aligned); flags:
+ *                            CAVB200_FKT_RECORD appends a record against the references stored so far,
+ *                            CAVB200_FKT_ADD_REFERENCE afterwards stores this frame's rho as the next reference.
+ *                            Asynchronous, stream-ordered.  N == 0 gives rho = 0.  cudaErrorInvalidValue for
+ *                            flags == 0, ADD_REFERENCE with max_references already stored, or a handle without open.
+ *   cavb200_fkt_track_read   newest min(max_records, stored) records, oldest first; *total = records appended since
+ *                            open.  Synchronises the stream. */
+#define CAVB200_FKT_RECORD 1u        /* append a record: F of every stored reference against this frame, and rho(t) */
+#define CAVB200_FKT_ADD_REFERENCE 2u /* afterwards, this frame's rho becomes the next stored reference              */
+int cavb200_fkt_track_open(cavb200_handle* h, const double* kvec_host, uint32_t K, uint32_t max_references,
+                           uint32_t capacity, uint32_t N);
+int cavb200_fkt_track_step(cavb200_handle* h, const double* pos, uint32_t N, uint64_t timestep, uint32_t flags,
+                           void* stream);
+int cavb200_fkt_track_read(cavb200_handle* h, double* out, uint32_t max_records, uint32_t* n_out, uint64_t* total,
+                           void* stream);
+
 /* ---- particle-sharded multi-GPU (one process per GPU) -------------------------------------------
  * New functionality (the reference never reduces across ranks, SURVEY.md 2.3): each rank holds a
  * contiguous block of particles; between the reduce pass and the apply pass the ranks combine

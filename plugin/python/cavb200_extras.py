@@ -61,3 +61,61 @@ def make_fused_method(simulation, filter, bussi, cavity_force, mode="rank1"):
     group = simulation.state._get_group(filter)
     return _cavitymd.TwoStepConstantVolumeCavity(simulation.state._cpp_sys_def, group, _cpp(bussi) if bussi is not None else None,
                                                  _cpp(cavity_force), mode)
+
+
+class FieldAutocorrelation:
+    """F(k,t) without snapshots, on the schedule of the reference's FieldAutocorrelationTracker.act
+    (src/cavitymd/analysis.py:380-414): reference 0 at construction, nothing at timestep 0, then every step a record of F
+    against every stored reference, and a new reference once `reference_interval_steps` have passed since the last one
+    while fewer than `max_references` are stored.  The density field rho(t) and F are formed on the device by the cavity
+    force's C++ object (fktOpen / fktStep / fktRead, include/cavb200.h); act() issues one asynchronous step and returns
+    nothing, read() brings back what was recorded since the previous read.
+
+    wavevectors: K x 3, e.g. the reference's hoomd.cavitymd.analysis.generate_fibonacci_sphere(n) * kmag.  cavity_force:
+    the attached CavityForce wrapper or its C++ object.  In the fused method's "one_launch" mode the positions are
+    complete after every launch (only the velocities lag half a kick), so act() needs no flush() of the method.
+    Constructing another tracker on the same force re-opens the device tracker and drops this one's references."""
+
+    def __init__(self, cavity_force, wavevectors, reference_interval_steps=10000, max_references=10, capacity=16384):
+        self._cpp_force = cavity_force if hasattr(cavity_force, "fktOpen") else _cpp(cavity_force)
+        self.wavevectors = [tuple(float(c) for c in k) for k in wavevectors]
+        self.K = len(self.wavevectors)
+        self.reference_interval_steps = reference_interval_steps
+        self.max_references = max_references
+        self.capacity = capacity
+        self._cpp_force.fktOpen(self.wavevectors, max_references, capacity)
+        self.reference_timesteps = []  # timestep of reference r
+        self.last_reference_step = 0
+        self._seen = 0
+        self._cpp_force.fktStep(0, False, True)
+        self.reference_timesteps.append(0)
+
+    def act(self, timestep):
+        if timestep == 0:
+            return
+        add = (len(self.reference_timesteps) < self.max_references
+               and timestep - self.last_reference_step >= self.reference_interval_steps)
+        self._cpp_force.fktStep(timestep, True, add)
+        if add:
+            self.reference_timesteps.append(timestep)
+            self.last_reference_step = timestep
+
+    def read(self):
+        """-> (rows, rho) of the records appended since the previous read (at most `capacity`, the newest): rows are
+        (reference number, timestep, lag in steps, F), record by record and reference by reference as act() of the
+        reference produces them; rho is float64[n_records, K, 2] ({re, im} of rho(t) per record)."""
+        _, total = self._cpp_force.fktRead(0)
+        records, total = self._cpp_force.fktRead(min(total - self._seen, self.capacity))
+        self._seen = total
+        return records_to_rows(records, self.reference_timesteps, self.max_references), \
+            records[:, 2 + self.max_references:].reshape(len(records), self.K, 2)
+
+
+def records_to_rows(records, reference_timesteps, max_references):
+    """Rows (reference number, timestep, lag, F) of F(k,t) tracker records (layout: include/cavb200.h)."""
+    rows = []
+    for rec in records:
+        t = int(rec[0])
+        for r in range(int(rec[1])):
+            rows.append((r, t, t - reference_timesteps[r], float(rec[2 + r])))
+    return rows

@@ -2,7 +2,9 @@
 #include "CavityForceComputeGPU.h"
 
 #include <cuda_runtime.h>
+#include <pybind11/numpy.h>
 
+#include <algorithm>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -208,6 +210,48 @@ pybind11::list CavityForceComputeGPU::trackRead(unsigned int max_records)
     return out;
     }
 
+void CavityForceComputeGPU::fktOpen(pybind11::object kvectors, unsigned int max_references, unsigned int capacity)
+    {
+    std::vector<double> k;
+    for (auto row : kvectors)
+        {
+        size_t c = 0;
+        for (auto v : row)
+            {
+            k.push_back(v.cast<double>());
+            c++;
+            }
+        if (c != 3)
+            throw std::invalid_argument("CavityForceComputeGPU::fktOpen: every wave vector needs 3 components");
+        }
+    check(cavb200_fkt_track_open(m_handle, k.data(), (uint32_t)(k.size() / 3), max_references, capacity, m_pdata->getN()),
+          "cavb200_fkt_track_open");
+    m_fkt_words = 2 + max_references + (unsigned int)(k.size() / 3) * 2;
+    }
+
+void CavityForceComputeGPU::fktStep(uint64_t timestep, bool record, bool add_reference)
+    {
+    // asynchronous on this object's stream, after whatever wrote the positions; the wrapped positions of every particle,
+    // photon included, as the reference's compute_density_field takes them
+    ArrayHandle<Scalar4> d_pos(m_pdata->getPositions(), access_location::device, access_mode::read);
+    const uint32_t flags = (record ? CAVB200_FKT_RECORD : 0u) | (add_reference ? CAVB200_FKT_ADD_REFERENCE : 0u);
+    check(cavb200_fkt_track_step(m_handle, reinterpret_cast<const double*>(d_pos.data), m_pdata->getN(), timestep, flags,
+                                 m_stream),
+          "cavb200_fkt_track_step");
+    }
+
+pybind11::tuple CavityForceComputeGPU::fktRead(unsigned int max_records)
+    {
+    const size_t words = m_fkt_words ? m_fkt_words : 1;
+    std::vector<double> buf((size_t)max_records * words + 1);
+    uint32_t n = 0;
+    uint64_t total = 0;
+    check(cavb200_fkt_track_read(m_handle, buf.data(), max_records, &n, &total, m_stream), "cavb200_fkt_track_read");
+    pybind11::array_t<double> out({(size_t)n, words});
+    std::copy(buf.begin(), buf.begin() + (size_t)n * words, out.mutable_data());
+    return pybind11::make_tuple(out, total);
+    }
+
 namespace detail
     {
 void export_CavityForceComputeGPU(pybind11::module& m)
@@ -231,7 +275,12 @@ void export_CavityForceComputeGPU(pybind11::module& m)
         .def("trackOpen", &CavityForceComputeGPU::trackOpen, pybind11::arg("capacity"))
         .def("trackSetReference", &CavityForceComputeGPU::trackSetReference)
         .def("trackRecord", &CavityForceComputeGPU::trackRecord, pybind11::arg("timestep"))
-        .def("trackRead", &CavityForceComputeGPU::trackRead, pybind11::arg("max_records"));
+        .def("trackRead", &CavityForceComputeGPU::trackRead, pybind11::arg("max_records"))
+        .def("fktOpen", &CavityForceComputeGPU::fktOpen, pybind11::arg("kvectors"), pybind11::arg("max_references"),
+             pybind11::arg("capacity"))
+        .def("fktStep", &CavityForceComputeGPU::fktStep, pybind11::arg("timestep"), pybind11::arg("record"),
+             pybind11::arg("add_reference"))
+        .def("fktRead", &CavityForceComputeGPU::fktRead, pybind11::arg("max_records"));
     }
     } // namespace detail
     } // namespace cavitymd

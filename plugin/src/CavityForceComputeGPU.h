@@ -57,6 +57,15 @@ class PYBIND11_EXPORT CavityForceComputeGPU : public ForceCompute
     //! newest min(max_records, stored) records, oldest first: list of 16-tuples (layout: include/cavb200.h)
     pybind11::list trackRead(unsigned int max_records);
 
+    //! F(k,t) without snapshots: what FieldAutocorrelationTracker.act of the reference gets from a cpu_local_snapshot and
+    //! K NumPy passes every step (src/cavitymd/analysis.py:260-418) is formed on the device on this object's handle and
+    //! stream, one record per step {timestep, n_refs, F per reference, rho(t)} (layout: include/cavb200.h).
+    //! kvectors: K rows of 3 numbers.  fktOpen blocks and drops every stored reference; fktStep is asynchronous and reads
+    //! the current positions; fktRead returns (records float64[n, 2 + max_references + 2K] oldest first, total appended).
+    void fktOpen(pybind11::object kvectors, unsigned int max_references, unsigned int capacity);
+    void fktStep(uint64_t timestep, bool record, bool add_reference);
+    pybind11::tuple fktRead(unsigned int max_records);
+
     //! Used by TwoStepConstantVolumeCavity (SURVEY.md 8f.1/8f.2).  mode 0: back to normal (own handle, forces stored).
     //! mode 1: rank-1 -- the dipole reduce runs on the integration method's handle `h` and NOTHING is written per
     //! particle: m_force stays zero, the method's kicks form F_i = (-g c_i) Dq from the charge
@@ -81,6 +90,7 @@ class PYBIND11_EXPORT CavityForceComputeGPU : public ForceCompute
     int m_mode = 0;
     bool m_integrator_reduced = false;
     bool m_zeroed = false;
+    unsigned int m_fkt_words = 0; //!< doubles per F(k,t) record (0: fktOpen not called)
     };
 
 namespace detail
