@@ -113,6 +113,8 @@ _SIGNATURES = {
     "cavb200_track_open": (C.c_int, [_vp, _u32]),
     "cavb200_track_set_reference": (C.c_int, [_vp, _vp]),
     "cavb200_track_record": (C.c_int, [_vp, _u64, _vp, _u32, _vp]),
+    "cavb200_track_set_reference_from": (C.c_int, [_vp, _vp, _vp]),
+    "cavb200_track_record_from": (C.c_int, [_vp, _vp, _vp, _u64, _vp, _u32, _u32, _vp]),
     "cavb200_track_read": (C.c_int, [_vp, _dp, _u32, C.POINTER(_u32), C.POINTER(_u64), _vp]),
     "cavb200_rhok": (C.c_int, [_vp, _vp, _u32, _u64, _u32, _u32, _vp, _u32, _vp, _vp]),
     "cavb200_rhok_f32": (C.c_int, [_vp, _vp, _u64, _u32, _u32, _vp, _u32, _vp, _vp]),
@@ -582,8 +584,18 @@ class Handle:
     def track_set_reference(self, stream=None):
         check(self.lib.cavb200_track_set_reference(self.h, stream), "cavb200_track_set_reference")
 
+    TRACK_VELOCITIES_PENDING = 1  # CAVB200_TRACK_VELOCITIES_PENDING
+
+    def track_set_reference_from(self, src: "Handle", stream=None):
+        check(self.lib.cavb200_track_set_reference_from(self.h, src.h, stream), "cavb200_track_set_reference_from")
+
     def track_record(self, timestep: int, vel, N: int, stream=None):
         check(self.lib.cavb200_track_record(self.h, timestep, _ptr(vel), N, stream), "cavb200_track_record")
+
+    def track_record_from(self, force_src: "Handle", bussi_src, timestep: int, vel, N: int, flags: int = 0, stream=None):
+        """bussi_src: the Handle that ran the thermostat, or None ([12..14] NaN)."""
+        check(self.lib.cavb200_track_record_from(self.h, force_src.h, bussi_src.h if bussi_src is not None else None,
+                                                 timestep, _ptr(vel), N, flags, stream), "cavb200_track_record_from")
 
     def track_read(self, max_records: int, stream=None):
         """-> (records float64[n, 16] oldest first, total appended since open)"""

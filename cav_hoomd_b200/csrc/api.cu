@@ -292,6 +292,7 @@ int cavb200_force(cavb200_handle* h, const double* pos, const double* charge, co
     int rc = fill_force(f, pos, charge, image, force, N, Lx, Ly, Lz, L_typeid, params, 0);
     if (rc)
         return rc;
+    h->index_offset = 0;
     return launch_hotpath(h, &f, nullptr, (cudaStream_t)stream);
     }
 
@@ -308,6 +309,7 @@ int cavb200_force_rank1(cavb200_handle* h, const double* pos, const double* char
     int rc = fill_force(f, pos, charge, image, nullptr, N, Lx, Ly, Lz, L_typeid, params, 0, false);
     if (rc)
         return rc;
+    h->index_offset = 0;
     return launch_hotpath(h, &f, nullptr, (cudaStream_t)stream);
     }
 
@@ -426,6 +428,7 @@ int cavb200_step(cavb200_handle* h, const double* pos, const double* charge, con
     int rc = fill_force(f, pos, charge, image, force, N, Lx, Ly, Lz, L_typeid, params, 0);
     if (rc)
         return rc;
+    h->index_offset = 0;
     if (bussi->deltaT == 0.0)
         return launch_hotpath(h, &f, nullptr, (cudaStream_t)stream);
     BussiIn b;

@@ -145,6 +145,9 @@ struct cavb200_handle
     // device-side tracker ring (track.cu): records | reference dipole | counter
     double* track_ring;
     uint64_t track_capacity;
+    // global index of this handle's particle 0 in the last force result: the index_offset of cavb200_shard_step, 0 after
+    // every other call that reduces the dipole.  The tracker maps the (global) photon index back to the local array.
+    uint64_t index_offset;
     // F(k,t) workspace
     double* rhok_partials;
     uint64_t rhok_partials_bytes;

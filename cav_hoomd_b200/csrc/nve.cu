@@ -940,6 +940,7 @@ static int md_args(MdArgs& a, cavb200_handle* h, const double* pos, const double
     a.fnew = ForceIn();
     if (const int rc = fill_force(a.fnew, pos, charge, image, nullptr, N, Lx, Ly, Lz, L_typeid, params, 0, false))
         return rc;
+    h->index_offset = 0;
     a.b = harness_bussi(group_first, n_group, bussi);
     a.r = rank1_in(h, charge, pos, L_typeid, params->couplstr);
     a.w = wrap ? WrapIn{const_cast<int32_t*>(image), Lx, Ly, Lz} : WrapIn();

@@ -491,6 +491,7 @@ int cavb200_shard_step(cavb200_handle* h, const double* pos, const double* charg
     b.rescale = bussi->deltaT != 0.0;
     b.stream_st = (uint64_t)n_group * 116ull > (63ull << 20); // as api.cu fill_bussi
     fill_bussi_constants(b, bussi);
+    h->index_offset = index_offset;
     return launch_shard_step(h, &f, &b, (cudaStream_t)stream);
     }
     }

@@ -12,13 +12,18 @@
 
 namespace cavb
     {
-// One record = CAVB200_TRACK_WORDS doubles (include/cavb200.h documents the layout).
-__global__ void k_track_record(const Scalars* __restrict__ sc, const double4* __restrict__ vel, uint32_t N,
-                               double timestep, const double* __restrict__ ref, double* __restrict__ ring,
+// One record = CAVB200_TRACK_WORDS doubles (include/cavb200.h documents the layout).  sc: the Scalars of the handle that
+// holds the force result; sb: those of the handle that ran the thermostat (nullptr: unknown, [12..14] are NaN); offset:
+// the global index of vel[0], so that the photon's (global) index finds its row in a rank's local array.
+__global__ void k_track_record(const Scalars* __restrict__ sc, const Scalars* __restrict__ sb, const double4* __restrict__ vel,
+                               uint32_t N, unsigned long long offset, uint32_t flags, double timestep,
+                               const double* __restrict__ ref, double* __restrict__ ring,
                                unsigned long long* __restrict__ count, unsigned long long capacity)
     {
     if (threadIdx.x != 0)
         return;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    const bool pending = flags & CAVB200_TRACK_VELOCITIES_PENDING;
     const unsigned long long n = *count;
     double* r = ring + (n % capacity) * CAVB200_TRACK_WORDS;
     r[0] = timestep;
@@ -36,16 +41,17 @@ __global__ void k_track_record(const Scalars* __restrict__ sc, const double4* __
     // cavity-mode kinetic energy 1/2 m |v|^2 of the photon (analysis.py:1352-1354)
     double ke_ph = 0.0;
     const long long ph = sc->photon_idx;
-    if (vel && ph >= 0 && (unsigned long long)ph < N)
+    const unsigned long long local = (unsigned long long)ph - offset;
+    if (vel && ph >= 0 && (unsigned long long)ph >= offset && local < N)
         {
-        const double4 v = vel[ph];
+        const double4 v = vel[local];
         const double v2 = __dadd_rn(__dadd_rn(__dmul_rn(v.x, v.x), __dmul_rn(v.y, v.y)), __dmul_rn(v.z, v.z));
         ke_ph = __dmul_rn(__dmul_rn(0.5, v.w), v2);
         }
-    r[11] = ke_ph;
-    r[12] = sc->ke;
-    r[13] = sc->alpha;
-    r[14] = sc->cumulative;
+    r[11] = pending ? nan : ke_ph;
+    r[12] = sb && !pending ? sb->ke : nan;
+    r[13] = sb ? sb->alpha : nan;
+    r[14] = sb ? sb->cumulative : nan;
     r[15] = (double)ph;
     *count = n + 1;
     }
@@ -83,11 +89,32 @@ extern "C" int cavb200_track_open(cavb200_handle* h, uint32_t capacity)
 static double* track_ref(cavb200_handle* h) { return h->track_ring + (size_t)h->track_capacity * CAVB200_TRACK_WORDS; }
 static unsigned long long* track_counter(cavb200_handle* h) { return reinterpret_cast<unsigned long long*>(track_ref(h) + 4); }
 
+extern "C" int cavb200_track_set_reference_from(cavb200_handle* h, const cavb200_handle* src, void* stream)
+    {
+    if (!h || !h->track_ring || !src)
+        return (int)cudaErrorInvalidValue;
+    k_track_set_reference<<<1, 32, 0, (cudaStream_t)stream>>>(src->scalars, track_ref(h));
+    CAVB_CHECK(cudaGetLastError());
+    h->launches += 1;
+    return 0;
+    }
+
 extern "C" int cavb200_track_set_reference(cavb200_handle* h, void* stream)
     {
-    if (!h || !h->track_ring)
+    return cavb200_track_set_reference_from(h, h, stream);
+    }
+
+extern "C" int cavb200_track_record_from(cavb200_handle* h, const cavb200_handle* force_src, const cavb200_handle* bussi_src,
+                                         uint64_t timestep, const double* vel, uint32_t N, uint32_t flags, void* stream)
+    {
+    if (!h || !h->track_ring || !force_src || (flags & ~CAVB200_TRACK_VELOCITIES_PENDING))
         return (int)cudaErrorInvalidValue;
-    k_track_set_reference<<<1, 32, 0, (cudaStream_t)stream>>>(h->scalars, track_ref(h));
+    if (vel && (reinterpret_cast<uintptr_t>(vel) & 31))
+        return (int)cudaErrorMisalignedAddress;
+    k_track_record<<<1, 32, 0, (cudaStream_t)stream>>>(force_src->scalars, bussi_src ? bussi_src->scalars : nullptr,
+                                                        reinterpret_cast<const double4*>(vel), N, force_src->index_offset,
+                                                        flags, (double)timestep, track_ref(h), h->track_ring,
+                                                        track_counter(h), h->track_capacity);
     CAVB_CHECK(cudaGetLastError());
     h->launches += 1;
     return 0;
@@ -95,15 +122,7 @@ extern "C" int cavb200_track_set_reference(cavb200_handle* h, void* stream)
 
 extern "C" int cavb200_track_record(cavb200_handle* h, uint64_t timestep, const double* vel, uint32_t N, void* stream)
     {
-    if (!h || !h->track_ring)
-        return (int)cudaErrorInvalidValue;
-    if (vel && (reinterpret_cast<uintptr_t>(vel) & 31))
-        return (int)cudaErrorMisalignedAddress;
-    k_track_record<<<1, 32, 0, (cudaStream_t)stream>>>(h->scalars, reinterpret_cast<const double4*>(vel), N, (double)timestep,
-                                                        track_ref(h), h->track_ring, track_counter(h), h->track_capacity);
-    CAVB_CHECK(cudaGetLastError());
-    h->launches += 1;
-    return 0;
+    return cavb200_track_record_from(h, h, h, timestep, vel, N, 0, stream);
     }
 
 extern "C" int cavb200_track_read(cavb200_handle* h, double* out, uint32_t max_records, uint32_t* n_out, uint64_t* total,

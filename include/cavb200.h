@@ -327,24 +327,41 @@ int cavb200_rank1_reindex(cavb200_handle* h, const double* pos, uint32_t N, uint
  * Replace the per-step cpu_local_snapshot of the reference's trackers (reference
  * src/cavitymd/analysis.py:188,234 AutocorrelationTracker / DipoleAutocorrelation, :1327
  * CavityModeTracker, :535,578 EnergyTracker) by a 128-byte record per step, appended on the device from
- * the results the last cavb200_force* / cavb200_bussi* / nvt step left there; the host reads the ring
- * once per output period.  Record layout (CAVB200_TRACK_WORDS doubles):
+ * the results the last cavb200_force* / cavb200_bussi* / nvt / md / shard step left there; the host reads the ring
+ * once per output period.  Record layout (CAVB200_TRACK_WORDS doubles), with "the force handle" the handle whose last
+ * call reduced the dipole and "the thermostat handle" the one whose last call published KE / alpha:
  *   [0] timestep   [1..3] total dipole d = sum_i q_i r~_i (compute_total_dipole_moment, :18-31; the photon
  *   is excluded, which is the same number whenever its charge is 0, examples/05_advanced_run.py:502)
  *   [4..6] photon coordinate q (unwrapped)   [7..9] harmonic, coupling, dipole-self energy
- *   [10] C(t) = d(ref) . d(t) (:222-224)   [11] cavity-mode kinetic energy 1/2 m|v|^2 of the photon (:1352-1354;
- *   0 if vel == NULL or there is no photon)   [12] group kinetic energy   [13] alpha   [14] cumulative
- *   reservoir energy   [15] photon index (-1: none; the cavity force then computes nothing, reference
- *   src/CavityForceCompute.cc:149-156, and [1..11] are 0).
- *   cavb200_track_open(capacity)   allocate / reset the ring (oldest records are overwritten when full)
+ *   -- [1..3] and [7..9] bit for bit what cavb200_force_read of the force handle returns
+ *   [10] C(t) = d(ref) . d(t) = fl(fl(fl(ref_x d_x) + ref_y d_y) + ref_z d_z), no fused multiply-add (:222-224)
+ *   [11] cavity-mode kinetic energy fl(fl(0.5 m) fl(fl(v_x^2 + v_y^2) + v_z^2)) of the photon's row of `vel` (:1352-1354);
+ *   0 if vel == NULL, there is no photon, or the photon is not among this rank's N rows
+ *   [12] group kinetic energy   [13] alpha   [14] cumulative reservoir energy -- bit for bit cavb200_bussi_read of the
+ *   thermostat handle; NaN when no thermostat handle is given
+ *   [15] photon index, GLOBAL (after cavb200_shard_step: index_offset + local row; -1: none on this rank -- the cavity
+ *   force then computes nothing, reference src/CavityForceCompute.cc:149-156, and [1..11] are 0).
+ *   cavb200_track_open(capacity)   allocate / reset the ring and the reference (oldest records are overwritten when full)
  *   cavb200_track_set_reference    d(ref) <- current dipole (_initialize_reference / _start_new_reference)
- *   cavb200_track_record           append one record; asynchronous, stream-ordered after the step's kernels
+ *   cavb200_track_record           append one record; asynchronous, stream-ordered after the step's kernels.  The force
+ *                                  handle and the thermostat handle are h itself.
+ *   cavb200_track_record_from      the same into h's ring, with the dipole, q, energies and photon index read from
+ *                                  force_src and [12..14] from bussi_src (NULL: NaN) -- for a caller whose force and
+ *                                  thermostat run on other handles than the one that keeps the ring.  The photon's row
+ *                                  of `vel` is photon index - index_offset of force_src's last call.
+ *                                  flags CAVB200_TRACK_VELOCITIES_PENDING: `vel` is half a kick short of the step (the
+ *                                  deferred second half kick of cavb200_md_step_fused); [11] and [12] are NaN.
+ *   cavb200_track_set_reference_from   d(ref) <- current dipole of src
  *   cavb200_track_read             newest min(max_records, stored) records, oldest first; *total = records
  *                                  appended since open.  Synchronises the stream. */
 #define CAVB200_TRACK_WORDS 16
+#define CAVB200_TRACK_VELOCITIES_PENDING 1u
 int cavb200_track_open(cavb200_handle* h, uint32_t capacity);
 int cavb200_track_set_reference(cavb200_handle* h, void* stream);
+int cavb200_track_set_reference_from(cavb200_handle* h, const cavb200_handle* src, void* stream);
 int cavb200_track_record(cavb200_handle* h, uint64_t timestep, const double* vel, uint32_t N, void* stream);
+int cavb200_track_record_from(cavb200_handle* h, const cavb200_handle* force_src, const cavb200_handle* bussi_src,
+                              uint64_t timestep, const double* vel, uint32_t N, uint32_t flags, void* stream);
 int cavb200_track_read(cavb200_handle* h, double* out, uint32_t max_records, uint32_t* n_out, uint64_t* total,
                        void* stream);
 

@@ -181,16 +181,20 @@ void CavityForceComputeGPU::trackOpen(unsigned int capacity)
 
 void CavityForceComputeGPU::trackSetReference()
     {
-    check(cavb200_track_set_reference(m_handle, m_stream), "cavb200_track_set_reference");
+    check(cavb200_track_set_reference_from(m_handle, m_ext_handle ? m_ext_handle : m_handle, m_stream),
+          "cavb200_track_set_reference_from");
     }
 
 void CavityForceComputeGPU::trackRecord(uint64_t timestep)
     {
-    // asynchronous, ordered after this step's force kernel on HOOMD's stream; the photon's kinetic energy needs
-    // the velocities, everything else is already on the device
+    // asynchronous, ordered after this step's kernels on HOOMD's stream; the photon's kinetic energy needs the
+    // velocities, everything else is already on the device: the force result on the handle that computed it, KE / alpha
+    // on the handle the thermostat ran on
     ArrayHandle<Scalar4> d_vel(m_pdata->getVelocities(), access_location::device, access_mode::read);
-    check(cavb200_track_record(m_handle, timestep, reinterpret_cast<const double*>(d_vel.data), m_pdata->getN(), m_stream),
-          "cavb200_track_record");
+    check(cavb200_track_record_from(m_handle, m_ext_handle ? m_ext_handle : m_handle, m_bussi_handle, timestep,
+                                    reinterpret_cast<const double*>(d_vel.data), m_pdata->getN(),
+                                    m_vel_pending ? CAVB200_TRACK_VELOCITIES_PENDING : 0u, m_stream),
+          "cavb200_track_record_from");
     }
 
 pybind11::list CavityForceComputeGPU::trackRead(unsigned int max_records)

@@ -51,6 +51,11 @@ class PYBIND11_EXPORT CavityForceComputeGPU : public ForceCompute
     //! Device-side trackers (SURVEY.md 8f.4): what DipoleAutocorrelation / CavityModeTracker / EnergyTracker of the
     //! reference get from a full cpu_local_snapshot every step (src/cavitymd/analysis.py:188,234,535,578,1327) is
     //! appended on the device, one 128-byte record per call, and read back once per output period.
+    //! The ring lives on this object's own handle, so attaching or detaching an integration method keeps a run's records.
+    //! A record reads the dipole, q, energies and photon index of the handle that computes the force (the method's in the
+    //! rank-1 modes) and [12..14] of the handle that ran the thermostat (the method's; NaN with no method attached, since
+    //! this object cannot know a thermostat of its own).  While the method's one_launch mode holds a second half kick
+    //! back, [11] and [12] are NaN: they need the velocities of the full step (flush() first).
     void trackOpen(unsigned int capacity);
     void trackSetReference();
     void trackRecord(uint64_t timestep);
@@ -73,6 +78,11 @@ class PYBIND11_EXPORT CavityForceComputeGPU : public ForceCompute
     //! dipole of the new positions, so computeForces only runs the reduce until the method has taken over.
     void useHandle(cavb200_handle* h, int mode);
     void integratorHasReduced() { m_integrator_reduced = true; m_fresh = false; }
+    //! Used by TwoStepConstantVolumeCavity in every mode: the handle whose step kernels publish KE / alpha / reservoir
+    //! (nullptr: none), and whether the velocities are half a kick short of the step (one_launch between flushes).
+    void useThermostatHandle(cavb200_handle* h) { m_bussi_handle = h; }
+    cavb200_handle* thermostatHandle() const { return m_bussi_handle; }
+    void setVelocitiesPending(bool pending) { m_vel_pending = pending; }
     const cavb200_params& params() const { return m_params; }
 
     protected:
@@ -87,6 +97,8 @@ class PYBIND11_EXPORT CavityForceComputeGPU : public ForceCompute
     bool m_fresh; //!< host copies are current
     void* m_stream = nullptr;
     cavb200_handle* m_ext_handle = nullptr; //!< the integration method's handle (rank-1 modes), not owned
+    cavb200_handle* m_bussi_handle = nullptr; //!< the handle the thermostat runs on (the method's), not owned
+    bool m_vel_pending = false;             //!< one_launch: the velocities lack the deferred second half kick
     int m_mode = 0;
     bool m_integrator_reduced = false;
     bool m_zeroed = false;

@@ -45,6 +45,8 @@ TwoStepConstantVolumeCavity::TwoStepConstantVolumeCavity(std::shared_ptr<SystemD
         m_source->adoptHandle(m_handle);
     if (m_cavity && m_mode != STORED)
         m_cavity->useHandle(m_handle, m_mode == RANK1 ? 1 : 2);
+    if (m_cavity) // in every mode the step kernels publish KE / alpha / reservoir on this handle: the tracker reads them here
+        m_cavity->useThermostatHandle(m_handle);
     m_pdata->getParticleSortSignal().connect<TwoStepConstantVolumeCavity, &TwoStepConstantVolumeCavity::slotParticleSort>(this);
     }
 
@@ -56,6 +58,11 @@ TwoStepConstantVolumeCavity::~TwoStepConstantVolumeCavity()
         m_source->adoptHandle(nullptr);
     if (m_cavity && m_mode != STORED)
         m_cavity->useHandle(nullptr, 0);
+    if (m_cavity && m_cavity->thermostatHandle() == m_handle)
+        {
+        m_cavity->useThermostatHandle(nullptr);
+        m_cavity->setVelocitiesPending(false);
+        }
     cavb200_destroy(m_handle);
     }
 
@@ -303,6 +310,7 @@ void TwoStepConstantVolumeCavity::integrateStepTwo(uint64_t timestep)
         m_pending = true; // rides on the next step one (or flush())
         m_pending_bath = (bool)m_bath_group;
         m_pending_args = bath;
+        m_cavity->setVelocitiesPending(true); // the tracker must not record the half-kicked velocities as the step's
         return;
         }
     unsigned int first = 0, n = 0;
@@ -363,6 +371,7 @@ void TwoStepConstantVolumeCavity::flush()
               "cavb200_nvt_step_two_rank1");
     m_pending = false;
     m_pending_bath = false;
+    m_cavity->setVelocitiesPending(false);
     // the velocities are now complete, but the next step one must not redo this half kick: restart from md_step_one
     }
 

@@ -18,7 +18,8 @@ def header_symbols():
 def test_header_declares_the_expected_entry_points():
     syms = header_symbols()
     for must in ("cavb200_create", "cavb200_force", "cavb200_force_read", "cavb200_bussi", "cavb200_bussi_ke",
-                 "cavb200_step", "cavb200_step_host", "cavb200_rhok", "cavb200_fkt", "cavb200_shard_step"):
+                 "cavb200_step", "cavb200_step_host", "cavb200_rhok", "cavb200_fkt", "cavb200_shard_step",
+                 "cavb200_track_record", "cavb200_track_record_from", "cavb200_track_set_reference_from"):
         assert must in syms
 
 

@@ -2,9 +2,11 @@
 """tools/sass_compare.py OLD.so NEW.so -- compare the machine code (cuobjdump -sass) of every kernel of two
 libcavb200.so builds, e.g. the parent commit's and this one's.
 
-Instructions are compared without addresses and encodings.  Kernels are matched by demangled name; a harness kernel
-that gained a trailing bool template parameter (nve.cu: MASK, BATH) and a trailing parameter of a new type is matched to
-its parent by dropping both when the new parameter is false.  Prints SAME / DIFF / NEW / GONE lines and a count."""
+Instructions are compared without addresses and encodings.  Kernels are matched by demangled name; a kernel whose
+parameter list changed is matched by its name without the parameter list when that is unique (k_track_record gained
+parameters and a flags word); a harness kernel that gained a trailing bool template parameter (nve.cu: MASK, BATH) and a
+trailing parameter of a new type is matched to its parent by dropping both when the new parameter is false.  Prints
+SAME / DIFF / NEW / GONE lines and a count."""
 import re
 import subprocess
 import sys
@@ -45,8 +47,14 @@ def main():
     old, new = kernels(sys.argv[1]), kernels(sys.argv[2])
     same = diff = 0
     matched = set()
+    by_stem = {}
+    for p in old:
+        by_stem.setdefault(p.split("(")[0], []).append(p)
     for n, body in sorted(new.items()):
-        p = parent_name(n)
+        p = n
+        if p not in old:
+            stem = by_stem.get(n.split("(")[0], [])
+            p = stem[0] if len(stem) == 1 and stem[0] not in new else parent_name(n)
         if p is None:
             print(f"NEW   {n.split('(')[0]}  ({len(body)} instructions)")
             continue
